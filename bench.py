@@ -3,6 +3,7 @@ bench.py — CV model fits/sec of the sGLM hot path on B200 (BASELINE.json metri
 
     python bench.py --gpus N --steps K --warmup W          (N>1: launched by torch.distributed.run)
     python bench.py --impl reference ...                   (CPU arm: the reference's own path)
+    python bench.py ... --dump-outputs DIR                 (also write the last timed step's results as DIR/*.npy)
 
 One "step" = one pass of the hot path over one synthetic session:
     lag/shift gather  (T x P base signals  ->  T x C design, NaN edge rows dropped)
@@ -57,7 +58,8 @@ FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustain
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3, help="timed steps of every timed leg (device-resident, end to end, "
+                                                         "--impl reference); the cpu_baseline leg times one sample step")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--mode", default="grid", choices=["grid", "sessions"])
@@ -80,7 +82,14 @@ def parse_args():
     ap.add_argument("--no-probes", action="store_true")
     ap.add_argument("--cpu-sample-T", type=int, default=0, help="rows of the CPU sample (0: 40000 for --impl reference, "
                                                                "16000 for the cpu_baseline leg)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last device-resident step returned (per parameter set: "
+                         "fold and refit coefficients, intercepts, scores; the selection) as DIR/<name>.npy in float64, "
+                         "at most 64 MB (a seeded sample of the parameter sets beyond that)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload(args):
@@ -272,6 +281,38 @@ def measure_probes(nat, torch):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 * 2**20
+DUMP_FIELDS = ("cv_coefs", "cv_intercepts", "cv_scores_train", "cv_scores_test", "cv_mean_score_train", "cv_mean_score",
+               "cv_std_score", "cv_R2_score", "cv_mse_score")
+
+
+def dump_outputs(res, out_dir):
+    """Writes the result dict of one CV grid step as float64 DIR/<name>.npy, row i = parameter set set_index[i] of the
+    grid: the DUMP_FIELDS of every set (cv_coefs stacked to sets x C x folds), the refit's coef / intercept, and the
+    selection (best_set, best_score, best_score_std).  Two builds run with the same arguments get the same inputs, so
+    their dumps compare output for output.  Past DUMP_LIMIT_BYTES a fixed, seeded sample of the sets is written."""
+    full = res["full_cv_results"]
+
+    def row(r):
+        return [r[k] for k in DUMP_FIELDS] + [r["model"].coef_, r["model"].intercept_]
+    names = list(DUMP_FIELDS) + ["coef", "intercept"]
+    n = len(full)
+    row_bytes = 8 * (1 + sum(np.size(v) for v in row(full[0])))       # + its set_index entry
+    k = min(n, (DUMP_LIMIT_BYTES - 4096) // row_bytes)
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    rows = [row(full[i]) for i in idx]
+    out = {name: np.stack([np.asarray(r[j], dtype=np.float64) for r in rows]) for j, name in enumerate(names)}
+    out["set_index"] = idx.astype(np.float64)
+    out["best_set"] = np.float64([r["glm_kwargs"] for r in full].index(res["best_params"]))
+    out["best_score"] = np.float64(res["best_score"])
+    out["best_score_std"] = np.float64(res["best_score_std"])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    mb = sum(a.nbytes for a in out.values()) / 2**20
+    sys.stderr.write(f"[dump] {len(out)} arrays, {mb:.1f} MB, {k} of {n} parameter sets -> {out_dir}\n")
+
+
 def main():
     args = parse_args()
     # stdout carries exactly ONE JSON line: everything else written to file descriptor 1 by libraries (NCCL prints its
@@ -292,7 +333,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps, warmup = max(1, min(args.steps, 2)), min(args.warmup, 1)
+        steps, warmup = args.steps, min(args.warmup, 1)
         Ts = args.cpu_sample_T or 40_000
         v, v_sample, sec, sample, detail = cpu_reference_run(args, Ts, (0.0, 0.25, 0.5, 1.0), 3, steps, warmup)
         cfg = config_dict(args, n_gpus, mode)
@@ -459,6 +500,8 @@ def main():
     nat.enable_timing(False)
     launches = nat.launches() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(res, args.dump_outputs)
     n_sessions = world * args.sessions_per_gpu if mode == "sessions" else 1
     value = fits_per_step * args.steps * n_sessions / (total_ms / 1e3)
 
@@ -617,7 +660,7 @@ def main():
     e2e = None
     if not args.no_e2e and step_e2e is not None:
         step_e2e()
-        e2e_steps = max(1, min(args.steps, 2))
+        e2e_steps = args.steps
         e2e_ms, res_e = timed(step_e2e, e2e_steps)
         h2d = X0_pin.numel() * 8 + y_pin.numel() * 8 + sum((a.numel() + b.numel()) * 8 for a, b in folds_pin)
         d2h = 0
