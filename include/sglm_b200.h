@@ -387,6 +387,28 @@ int sglm_poisson_irls_prepare_f64(const double *X, int64_t ldx, const double *y,
                                   void *stream);
 
 /* ------------------------------------------------------------------------- *
+ * The same two passes for the Tweedie family of `power` with log link (scikit-learn
+ * TweedieRegressor(power=p) / HalfTweedieLoss; reference backend/sglm.py:112-117:
+ * 'Poisson' p = 1, 'Gamma' p = 2, 'Tweedie' any p).  power must be 1 or > 1, else
+ * SGLM_E_UNSUPPORTED before any CUDA call.  power = 1 computes exactly what
+ * sglm_score_f64 (link 1) / sglm_poisson_irls_prepare_f64 compute.
+ *   score_glm:         sums[0..7] = { n, sum r^2, sum y, sum y^2, s4, s5, s6, sum r },
+ *                      r = y - mu; the deviance terms s4..s6 are
+ *                        p = 1: { y*eta, mu, y log y };  p = 2: { eta, y/mu, log y };
+ *                        other p: { y mu^(1-p), mu^(2-p), y^(2-p) }.
+ *   glm_irls_prepare:  weight[t] = rw[t] * mu^(2-p) (Fisher weight), z[t] = eta + (y-mu)/mu,
+ *                      sums[0..3] = { sum rw*loss, sum weight, sum rw, sum rw*y } with the
+ *                      unit loss mu - y eta (p = 1), eta + y/mu (p = 2),
+ *                      mu^(2-p)/(2-p) - y mu^(1-p)/(1-p) (other p).
+ * ------------------------------------------------------------------------- */
+int sglm_score_glm_f64(const double *X, int64_t ldx, const double *y, const double *rw, int64_t T,
+                       int32_t C, const double *w, const double *b_dev, double power, double *resid,
+                       double *sums, void *workspace, void *stream);
+int sglm_glm_irls_prepare_f64(const double *X, int64_t ldx, const double *y, const double *rw,
+                              int64_t T, int32_t C, const double *w, const double *b_dev, double power,
+                              double *weight, double *z, double *sums, void *workspace, void *stream);
+
+/* ------------------------------------------------------------------------- *
  * Steps either side of the lag builder, for data already on the device (SURVEY.md §8f-3):
  *   col_moments + zscore_apply : sglm_pp.zscore (backend/sglm_pp.py:105-118): (X - mean) / std per column; ddof 0 =
  *                   numpy std (ndarray input), 1 = pandas std (DataFrame input); skipna as pandas does.
@@ -443,6 +465,13 @@ int sglm_pb_epilogue_f64(double *Eta, int64_t ldb, int32_t n_models, int64_t T, 
                          const int32_t *ycol, const double *RW, int64_t ldrw, const int32_t *rw_a,
                          const int32_t *rw_b, const double *b, const int32_t *status, int32_t mode, double *sums,
                          void *workspace, size_t workspace_bytes, void *stream);
+/* sglm_pb_epilogue_f64 for the Tweedie family of `power` (1, or > 1 — else SGLM_E_UNSUPPORTED before any CUDA call;
+ * log link): mode 0 writes R = rw dloss/deta = rw mu^(1-p) (mu - y) and sums [B][4] = {sum rw loss, sum rw mu^(2-p),
+ * sum rw, sum R}; mode 1 the sglm_score_glm_f64 sums.  power = 1 is sglm_pb_epilogue_f64. */
+int sglm_glm_epilogue_f64(double *Eta, int64_t ldb, int32_t n_models, int64_t T, const double *Y, int64_t ldy,
+                          const int32_t *ycol, const double *RW, int64_t ldrw, const int32_t *rw_a,
+                          const int32_t *rw_b, const double *b, const int32_t *status, double power, int32_t mode,
+                          double *sums, void *workspace, size_t workspace_bytes, void *stream);
 int sglm_pb_state_words(void);
 int sglm_pb_step_f64(const uint64_t *state_host, const double *const *L_of, void *stream);
 

@@ -1006,8 +1006,9 @@ def predict(Xd, coef, intercept, link=0):
     return out
 
 
-def score_sums(Xd, yd, coef, intercept, link=0, rw=None, want_resid=False):
-    """Fused pass: {n, sum r^2, sum y, sum y^2, sum y*eta, sum mu, sum y log y, sum r} (host)."""
+def score_sums(Xd, yd, coef, intercept, link=0, rw=None, want_resid=False, power=None):
+    """Fused pass: {n, sum r^2, sum y, sum y^2, sum y*eta, sum mu, sum y log y, sum r} (host).  With `power` (log link):
+    the Tweedie family's deviance terms in slots 4..6 (sglm_score_glm_f64), the input of tweedie_d2_from_sums."""
     torch = nat.require_cuda()
     T, C = Xd.shape
     w, b = _coef_dev(coef, intercept)
@@ -1016,8 +1017,12 @@ def score_sums(Xd, yd, coef, intercept, link=0, rw=None, want_resid=False):
     sums = _empty((8,))
     ws = torch.empty(nat.lib().sglm_score_workspace_bytes() // 8, dtype=torch.float64, device="cuda")
     resid = _empty((T,)) if want_resid else None
-    call("sglm_score_f64", ptr(Xd), row_stride(Xd), ptr(yd), ptr(rw), T, C, ptr(w), ptr(b), link, ptr(resid),
-         ptr(sums), ptr(ws), stream_ptr())
+    if power is None:
+        call("sglm_score_f64", ptr(Xd), row_stride(Xd), ptr(yd), ptr(rw), T, C, ptr(w), ptr(b), link, ptr(resid),
+             ptr(sums), ptr(ws), stream_ptr())
+    else:
+        call("sglm_score_glm_f64", ptr(Xd), row_stride(Xd), ptr(yd), ptr(rw), T, C, ptr(w), ptr(b), float(power),
+             ptr(resid), ptr(sums), ptr(ws), stream_ptr())
     return sums.cpu().numpy(), resid
 
 
@@ -1035,6 +1040,25 @@ def poisson_d2_from_sums(s):
     dev = 2.0 * (sylogy - sy_eta - sy + smu)
     ybar = sy / n
     dev_null = 2.0 * (sylogy - sy * np.log(ybar)) if ybar > 0 else 0.0
+    return float(1.0 - dev / dev_null)
+
+
+def tweedie_d2_from_sums(s, power):
+    """D^2 = 1 - dev/dev_null of the Tweedie family of `power` (log link; TweedieRegressor.score,
+    sklearn.metrics.d2_tweedie_score) from sums with the family's deviance terms {.., s4, s5, s6, ..}
+    (sglm_score_glm_f64, sglm_glm_epilogue_f64 mode 1); the null model is mu = mean(y)."""
+    if power == 1:
+        return poisson_d2_from_sums(s)
+    n, sy, s4, s5, s6 = s[0], s[2], s[4], s[5], s[6]
+    ybar = sy / n
+    if power == 2:
+        dev = 2.0 * (s4 - s6 + s5 - n)
+        dev_null = 2.0 * (n * np.log(ybar) - s6 + sy / ybar - n)
+    else:
+        p = float(power)
+        c = s6 / ((1.0 - p) * (2.0 - p))
+        dev = 2.0 * (c - s4 / (1.0 - p) + s5 / (2.0 - p))
+        dev_null = 2.0 * (c - sy * ybar ** (1.0 - p) / (1.0 - p) + n * ybar ** (2.0 - p) / (2.0 - p))
     return float(1.0 - dev / dev_null)
 
 
@@ -1208,33 +1232,41 @@ def poisson_irls(Xd, yd, alpha, fit_intercept=True, rw=None, max_iter=100, tol=1
 
 
 # --------------------------------------------------------------------------- #
-# (a9, batched) Poisson grid: all (fold, alpha) fits advance together (csrc/poisson_batch.cu)
+# (a9, batched) Poisson / Gamma / Tweedie grid: all (fold, alpha) fits advance together (csrc/poisson_batch.cu)
 # --------------------------------------------------------------------------- #
 PB_MAX_BATCH = 256       # models per batch (Eta is T x round_up(B, 64) doubles)
-last_poisson_batch = None    # diagnostics of the most recent batch: iterations, Hessian refreshes
+last_poisson_batch = None    # diagnostics of the most recent batch: iterations, Hessian refreshes, power
 
 
 class PoissonModel:
-    """One Poisson fit of a batch: penalty, row-weight vector (index into RW, -1 = all rows), response column."""
-    __slots__ = ("alpha", "fit_intercept", "rw", "ycol", "max_iter", "tol", "n_tot")
+    """One fit of a batch: penalty, row-weight vector (index into RW, -1 = all rows), response column, and an optional
+    start point (coef_init [C], intercept_init; default w = 0, b = log mean y)."""
+    __slots__ = ("alpha", "fit_intercept", "rw", "ycol", "max_iter", "tol", "n_tot", "coef_init", "intercept_init")
 
-    def __init__(self, alpha, fit_intercept=True, rw=-1, ycol=0, max_iter=100, tol=1e-4, n_tot=None):
+    def __init__(self, alpha, fit_intercept=True, rw=-1, ycol=0, max_iter=100, tol=1e-4, n_tot=None, coef_init=None,
+                 intercept_init=None):
         self.alpha, self.fit_intercept, self.rw, self.ycol = float(alpha), bool(fit_intercept), int(rw), int(ycol)
         self.max_iter, self.tol, self.n_tot = int(max_iter), float(tol), n_tot
+        self.coef_init, self.intercept_init = coef_init, intercept_init
 
 
-def _pb_hessian(Xd, y_col, rw_vec, w_ref, b_ref, fit_intercept, n_tot, use_tc):
-    """H~ = X' diag(rw mu_ref) X (centred on the weighted column means when an intercept is fitted) of one reference
-    model: the fused row pass gives the weights, the tcgen05 digit-plane Gram (large problems) or the fp64 DMMA Gram
-    the matrix.  Returns (Problem-like hess with Qc / xbar, h11 = sum of the weights as a device scalar)."""
+def _loss_name(power):
+    return "HalfPoissonLoss" if power == 1 else "HalfTweedieLoss"
+
+
+def _pb_hessian(Xd, y_col, rw_vec, w_ref, b_ref, fit_intercept, n_tot, use_tc, power=1.0):
+    """H~ = X' diag(rw v_ref) X (centred on the weighted column means when an intercept is fitted) with the Fisher
+    weights v_ref = mu_ref^(2-p) of one reference model: the fused row pass gives the weights, the tcgen05 digit-plane
+    Gram (large problems) or the fp64 DMMA Gram the matrix.  Returns (Problem-like hess with Qc / xbar, h11 = sum of
+    the weights as a device scalar)."""
     torch = nat.require_cuda()
     T, C = Xd.shape
     sums = _empty((8,))
     ws = torch.empty(nat.lib().sglm_score_workspace_bytes() // 8, dtype=torch.float64, device="cuda")
     weight = _empty((1, T))
     z = _empty((T, 1))
-    call("sglm_poisson_irls_prepare_f64", ptr(Xd), row_stride(Xd), ptr(y_col), ptr(rw_vec), T, C, ptr(w_ref), ptr(b_ref),
-         ptr(weight), ptr(z), ptr(sums), ptr(ws), stream_ptr())
+    call("sglm_glm_irls_prepare_f64", ptr(Xd), row_stride(Xd), ptr(y_col), ptr(rw_vec), T, C, ptr(w_ref), ptr(b_ref),
+         float(power), ptr(weight), ptr(z), ptr(sums), ptr(ws), stream_ptr())
     if use_tc:
         G = suffstats_tc_scaled(Xd, z, weight[0].sqrt(), POISSON_TC_PLANES)
     else:
@@ -1247,19 +1279,29 @@ def poisson_grid_batched(Xd, Yd, models, RW=None):
     """Fit every PoissonModel of `models` on (Xd, Yd[:, ycol]) with row weights RW[rw] — argmin mean(mu - y eta) +
     alpha/2 |w|^2 over the weighted rows — as ONE batched iteration (see csrc/poisson_batch.cu).  Returns
     (W [B, C] CUDA, b [B] CUDA, n_iter [B] host, status [B] host: 1 converged, 2 max_iter)."""
+    return tweedie_grid_batched(Xd, Yd, models, RW, 1.0)
+
+
+def tweedie_grid_batched(Xd, Yd, models, RW=None, power=1.0):
+    """poisson_grid_batched for the Tweedie family of `power` (1, or > 1; log link): argmin mean(l(y, eta)) +
+    alpha/2 |w|^2 with sklearn's HalfTweedieLoss l (p = 2: Gamma, whose Fisher Hessian X' diag(rw) X does not depend
+    on the iterate and is built once per fold)."""
     torch = nat.require_cuda()
     global last_poisson_batch
+    power = float(power)
+    if not (power == 1.0 or power > 1.0):
+        raise NotImplementedError(f"power={power}: the batched GLM solver covers power 1 and power > 1 (log link)")
     T, C = Xd.shape
     out_W, out_b, out_it, out_st = [], [], [], []
     diag = []
     for c0 in range(0, len(models), PB_MAX_BATCH):
-        Wb, bb, it, st, dg = _poisson_batch(Xd, Yd, models[c0:c0 + PB_MAX_BATCH], RW)
+        Wb, bb, it, st, dg = _poisson_batch(Xd, Yd, models[c0:c0 + PB_MAX_BATCH], RW, power)
         out_W.append(Wb); out_b.append(bb); out_it.append(it); out_st.append(st); diag.append(dg)
     last_poisson_batch = diag
     return torch.cat(out_W), torch.cat(out_b), np.concatenate(out_it), np.concatenate(out_st)
 
 
-def _poisson_batch(Xd, Yd, models, RW):
+def _poisson_batch(Xd, Yd, models, RW, power):
     torch = nat.require_cuda()
     T, C = Xd.shape
     B = len(models)
@@ -1274,15 +1316,22 @@ def _poisson_batch(Xd, Yd, models, RW):
                                       ((RW[rw] * Yd[:, yc]).sum() if rw >= 0 else Yd[:, yc].sum()),
                                       Yd[:, yc].min()]) for rw, yc in combos]).cpu().numpy()
     info = {k: v for k, v in zip(combos, stats)}
-    if any(v[2] < 0 for v in info.values()) or any(not (v[1] > 0) for v in info.values()):
-        raise ValueError("Some value(s) of y are out of the valid range of the loss 'HalfPoissonLoss'.")
+    if any(v[2] < 0 for v in info.values()) or any(not (v[1] > 0) for v in info.values()) or \
+            (power >= 2 and any(not (v[2] > 0) for v in info.values())):
+        raise ValueError(f"Some value(s) of y are out of the valid range of the loss '{_loss_name(power)}'.")
     n_tot = np.array([info[(m.rw, m.ycol)][0] for m in models])
     b0 = np.array([np.log(info[(m.rw, m.ycol)][1] / info[(m.rw, m.ycol)][0]) if m.fit_intercept else 0.0 for m in models])
     for yc in {m.ycol for m in models}:
         ycontig[yc] = Yd[:, yc].contiguous()
     # ---- state on the device
     f64, i32 = np.float64, np.int32
+    warm = [i for i, m in enumerate(models) if m.coef_init is not None]
+    for i in warm:
+        if models[i].fit_intercept and models[i].intercept_init is not None:
+            b0[i] = float(np.asarray(models[i].intercept_init, dtype=f64).reshape(-1)[0])
     W, Wprev, Wnew, rhs = (_zeros((B, ldw)) for _ in range(4))
+    for i in warm:
+        W[i, :C] = _dev(np.asarray(models[i].coef_init, dtype=f64).reshape(-1), f64)
     b = _dev(b0, f64)
     bprev, fprev, fcur, last_step, step_out = (_zeros((B,)) for _ in range(5))
     ratio_out = torch.ones(B, dtype=torch.float64, device="cuda")        # 1.0 = contraction not known yet
@@ -1327,7 +1376,8 @@ def _poisson_batch(Xd, Yd, models, RW):
         rw, fi = gkeys[g]
         idxs = groups[gkeys[g]]
         rw_vec = RW[rw] if rw >= 0 else None
-        hess, h11 = _pb_hessian(Xd, ycontig[models[ref].ycol], rw_vec, W[ref], b[ref:ref + 1], fi, float(n_tot[ref]), use_tc)
+        hess, h11 = _pb_hessian(Xd, ycontig[models[ref].ycol], rw_vec, W[ref], b[ref:ref + 1], fi, float(n_tot[ref]), use_tc,
+                                power)
         an = _dev([models[i].alpha * n_tot[i] for i in idxs], f64)
         wb = nat.lib().sglm_ridge_workspace_bytes(C, hess.ldq, len(idxs))
         work = torch.empty(wb // 8, dtype=torch.float64, device="cuda")
@@ -1349,10 +1399,11 @@ def _poisson_batch(Xd, Yd, models, RW):
             hscale[sel] = 1.0
             del borrowed[g]
 
-    # First step: every model starts from w = 0, b = log(mean y), where the Hessian is mean(y) * X'X over the model's
-    # rows.  A fold whose parameter sets also have a full-data model (the refit of every CV set) borrows that group's
-    # Hessian and factors for this one step, scaled by its share of sum(y) — 1 weighted Gram and 1 factorisation per
-    # alpha instead of one per (fold, alpha); its own Hessian follows with the refresh after the first step.
+    # First step: every model starts from w = 0, b = log(mean y), where the Hessian is mean(y)^(2-p) * X'X over the
+    # model's rows.  A fold whose parameter sets also have a full-data model (the refit of every CV set) borrows that
+    # group's Hessian and factors for this one step, scaled by n_f mean_f(y)^(2-p) / (n mean(y)^(2-p)) (p = 1: its
+    # share of sum(y)) — 1 weighted Gram and 1 factorisation per alpha instead of one per (fold, alpha); its own
+    # Hessian follows with the refresh after the first step.  Warm-started models start elsewhere and borrow nothing.
     hscale = torch.ones(B, dtype=torch.float64, device="cuda")
     borrowed = {}
     for g, (rw, fi) in enumerate(gkeys):
@@ -1361,7 +1412,7 @@ def _poisson_batch(Xd, Yd, models, RW):
         g0 = gkeys.index((-1, fi))
         by_alpha = {(models[i].alpha, models[i].ycol == 0): i for i in groups[gkeys[g0]]}
         pairs = [(i, by_alpha.get((models[i].alpha, True))) for i in groups[gkeys[g]]]
-        if all(j is not None for _, j in pairs):
+        if all(j is not None and models[i].coef_init is None and models[j].coef_init is None for i, j in pairs):
             borrowed[g] = (g0, pairs)
     for g in range(n_h):
         if g not in borrowed:
@@ -1372,7 +1423,13 @@ def _poisson_batch(Xd, Yd, models, RW):
         theirs = _dev([j for _, j in pairs], np.int64)
         hess_id[mine] = g0
         L_of[mine] = L_of[theirs]
-        share = np.array([info[(models[i].rw, models[i].ycol)][1] / info[(models[j].rw, models[j].ycol)][1] for i, j in pairs])
+        if power == 1:
+            share = np.array([info[(models[i].rw, models[i].ycol)][1] / info[(models[j].rw, models[j].ycol)][1] for i, j in pairs])
+        else:
+            def scale(k):
+                n_k, sy_k = info[(models[k].rw, models[k].ycol)][:2]
+                return n_k * (sy_k / n_k) ** (2.0 - power)
+            share = np.array([scale(i) / scale(j) for i, j in pairs])
         hscale[mine] = _dev(share, f64)
     n_words = nat.lib().sglm_pb_state_words()
     fields = [W, Wprev, Wnew, rhs, b, bprev, fprev, fcur, last_step, step_out, ratio_out, halv, n_iter, status, flag,
@@ -1388,8 +1445,8 @@ def _poisson_batch(Xd, Yd, models, RW):
     while it < max_rounds:
         Wt[:, :B] = W[:, :C].t()
         call("sglm_pb_eta_f64", ptr(Xd), row_stride(Xd), T, C, ptr(Wt), ldb, ptr(Eta), stream_ptr())
-        call("sglm_pb_epilogue_f64", ptr(Eta), ldb, B, T, ptr(Yd), ldy, ptr(ycol), RWp, ldrw, ptr(rw_a), None, ptr(b),
-             ptr(status), 0, ptr(sums), ptr(ep_ws), ep_ws.numel() * 8, stream_ptr())
+        call("sglm_glm_epilogue_f64", ptr(Eta), ldb, B, T, ptr(Yd), ldy, ptr(ycol), RWp, ldrw, ptr(rw_a), None, ptr(b),
+             ptr(status), power, 0, ptr(sums), ptr(ep_ws), ep_ws.numel() * 8, stream_ptr())
         call("sglm_pb_xt_r_f64", ptr(Xd), row_stride(Xd), T, C, ptr(Eta), ldb, ptr(Gw), ptr(xt_ws), xt_ws.numel() * 8,
              stream_ptr())
         call("sglm_pb_step_f64", state_p, ptr(L_of), stream_ptr())
@@ -1399,8 +1456,11 @@ def _poisson_batch(Xd, Yd, models, RW):
         if np.all(st_h != 0):
             break
         # refresh policy: after the first step (the start Hessian belongs to mu = const), then whenever the steps of a
-        # fold stop contracting by at least 3x per iteration; reference = the active model with the largest step
+        # fold stop contracting by at least 3x per iteration; reference = the active model with the largest step.
+        # Gamma (Fisher weight 1): a group's own Hessian is exact for every iterate, only a borrowed one is replaced.
         for g in range(n_h):
+            if power == 2 and g not in borrowed:
+                continue
             idxs = np.array(groups[gkeys[g]])
             act = idxs[st_h[idxs] == 0]
             if len(act) == 0 or n_refresh[g] >= 8:
@@ -1415,13 +1475,20 @@ def _poisson_batch(Xd, Yd, models, RW):
     st_f = status.cpu().numpy().astype(np.int64)
     st_f[st_f == 0] = 2
     return W[:, :C].contiguous(), b.clone(), n_it, st_f, dict(rounds=it, refreshes=dict(n_refresh), models=B,
-                                                              hessian_groups=n_h, tensor_core_hessian=bool(use_tc))
+                                                              hessian_groups=n_h, tensor_core_hessian=bool(use_tc),
+                                                              power=power)
 
 
 def poisson_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW):
     """Score sums of B fitted Poisson models in one pass over X: sums [B, 2, 8] (host) for the row weights rw_a /
     rw_b of each model (-1: all rows; rw_b = -2: none) — {n, sum r^2, sum y, sum y^2, sum y eta, sum mu,
     sum y log y, sum r}, the inputs of D^2 / -MSE / pooled R^2 (sglm_score_f64 semantics)."""
+    return tweedie_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW, 1.0)
+
+
+def tweedie_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW, power):
+    """poisson_scores_batched for the Tweedie family of `power`: slots 4..6 hold the family's deviance terms
+    (sglm_score_glm_f64 semantics), the input of tweedie_d2_from_sums."""
     torch = nat.require_cuda()
     T, C = Xd.shape
     B = W.shape[0]
@@ -1439,8 +1506,9 @@ def poisson_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW):
         # named tensors: a temporary freed inside the argument list would hand its block to the next allocation
         ids = _dev(np.stack([ycol[c0:c0 + n], rw_a[c0:c0 + n], rw_b[c0:c0 + n]]), np.int32)
         b_part = b[c0:c0 + n].contiguous()
-        call("sglm_pb_epilogue_f64", ptr(Eta), ldb, n, T, ptr(Yd), Yd.stride(0), ptr(ids[0]),
+        call("sglm_glm_epilogue_f64", ptr(Eta), ldb, n, T, ptr(Yd), Yd.stride(0), ptr(ids[0]),
              ptr(RW) if RW is not None else None, RW.stride(0) if RW is not None else 0,
-             ptr(ids[1]), ptr(ids[2]), ptr(b_part), None, 1, ptr(sums), ptr(ep_ws), ep_ws.numel() * 8, stream_ptr())
+             ptr(ids[1]), ptr(ids[2]), ptr(b_part), None, float(power), 1, ptr(sums), ptr(ep_ws), ep_ws.numel() * 8,
+             stream_ptr())
         out[c0:c0 + n] = sums.cpu().numpy().reshape(n, 2, 8)
     return out

@@ -1,7 +1,7 @@
 """
 Estimator objects behind `GLM.model` — the GPU counterparts of the scikit-learn classes
 the reference instantiates (backend/sglm.py:2, :95-130): LinearRegression, Ridge, Lasso,
-ElasticNet, TweedieRegressor(power=1).  Same constructor keywords (unknown keywords raise
+ElasticNet, TweedieRegressor (power 1 = Poisson, 2 = Gamma, any power > 1; log link).  Same constructor keywords (unknown keywords raise
 TypeError exactly as scikit-learn does, which is how stale kwargs such as `reg_lambda`
 fail in the reference), same fitted attributes (`coef_`, `intercept_`, `n_iter_`,
 `dual_gap_`), same `fit / predict / score`.  All arithmetic runs in libsglm_b200.so.
@@ -175,11 +175,17 @@ class Lasso(ElasticNet):
 
 
 class TweedieRegressor(_Base):
-    """Poisson GLM with log link (reference: backend/sglm.py:112-115 builds
-    TweedieRegressor(power=1); sklearn _glm/glm.py:185-339).  Fitted by IRLS/Newton on the
-    GPU to the optimum of  mean(mu - y*eta) + alpha/2 |w|^2 ; `score` is D^2."""
-    kind = "poisson"
+    """Tweedie GLM with log link (reference: backend/sglm.py:112-117 builds TweedieRegressor(power=1)
+    for 'Poisson', power=2 for 'Gamma', TweedieRegressor(**kwargs) for 'Tweedie'; sklearn
+    _glm/glm.py:185-339).  Fitted on the GPU to the optimum of  mean(l(y, eta)) + alpha/2 |w|^2
+    with sklearn's HalfTweedieLoss l — power 1 by IRLS/Newton, power > 1 by the batched solver
+    with one model; `score` is the family's D^2.  Power <= 0, 0 < power < 1 and the identity
+    link are not built."""
     _link = 1
+
+    @property
+    def kind(self):
+        return "poisson" if self.power == 1 else "tweedie"
 
     def __init__(self, *, power=0.0, alpha=1.0, fit_intercept=True, link="auto", solver="lbfgs",
                  max_iter=100, tol=1e-4, warm_start=False, verbose=0):
@@ -187,9 +193,16 @@ class TweedieRegressor(_Base):
         self.solver, self.max_iter, self.tol, self.warm_start, self.verbose = solver, max_iter, tol, warm_start, verbose
 
     def _check_family(self):
-        if self.power != 1 or self.link not in ("auto", "log"):
-            raise NotImplementedError("only the Poisson family with log link (power=1) is built on the GPU path; "
-                                      "Gamma/Tweedie(power!=1) are outside the hot-path scope")
+        if not (self.power == 1 or self.power > 1) or self.link not in ("auto", "log"):
+            raise NotImplementedError("the GPU path builds the Tweedie families with log link and power 1 (Poisson) "
+                                      "or power > 1 (Gamma, compound Poisson-Gamma, inverse Gaussian, ...); "
+                                      f"power={self.power!r}, link={self.link!r} is not built")
+
+    def _check_y(self, yd):
+        """scikit-learn's range check of HalfTweedieLoss: y >= 0 for power < 2, y > 0 for power >= 2."""
+        lo = float(yd.min().item()) if yd.numel() else 0.0
+        if not (lo >= 0) or (self.power >= 2 and not (lo > 0)):
+            raise ValueError(f"Some value(s) of y are out of the valid range of the loss '{eng._loss_name(self.power)}'.")
 
     def fit(self, X, y, sample_weight=None):
         if sample_weight is not None:
@@ -197,19 +210,34 @@ class TweedieRegressor(_Base):
         self._check_family()
         Xd, yd = eng.device_matrix(X), eng.device_vector(y)
         import torch
-        if bool((yd < 0).any().item()):
-            raise ValueError("Some value(s) of y are out of the valid range of the loss 'HalfPoissonLoss'.")
+        if self.power == 1:
+            if bool((yd < 0).any().item()):
+                raise ValueError("Some value(s) of y are out of the valid range of the loss 'HalfPoissonLoss'.")
+        else:
+            self._check_y(yd)
         if not bool(torch.isfinite(Xd).all().item()):
             raise ValueError("Input X contains NaN or infinity.")
         ci = getattr(self, "coef_", None) if self.warm_start else None
         ii = getattr(self, "intercept_", None) if self.warm_start else None
-        self.coef_, self.intercept_, self.n_iter_ = eng.poisson_irls(
-            Xd, yd, self.alpha, self.fit_intercept, None, self.max_iter, self.tol, ci, ii)
+        if self.power == 1:
+            self.coef_, self.intercept_, self.n_iter_ = eng.poisson_irls(
+                Xd, yd, self.alpha, self.fit_intercept, None, self.max_iter, self.tol, ci, ii)
+        else:
+            m = eng.PoissonModel(self.alpha, self.fit_intercept, max_iter=self.max_iter, tol=self.tol, coef_init=ci,
+                                 intercept_init=ii)
+            W, b, n_it, _ = eng.tweedie_grid_batched(Xd, yd[:, None], [m], None, self.power)
+            self.coef_ = W[0].cpu().numpy()
+            self.intercept_ = float(b[0].item()) if self.fit_intercept else 0.0
+            self.n_iter_ = int(n_it[0])
         self.n_features_in_ = Xd.shape[1]
         return self
 
     def score(self, X, y, sample_weight=None):
         self._check_family()
         Xd, yd = eng.device_matrix(X), eng.device_vector(y)
-        s, _ = eng.score_sums(Xd, yd, self.coef_, self.intercept_, 1)
-        return eng.poisson_d2_from_sums(s)
+        if self.power == 1:
+            s, _ = eng.score_sums(Xd, yd, self.coef_, self.intercept_, 1)
+            return eng.poisson_d2_from_sums(s)
+        self._check_y(yd)
+        s, _ = eng.score_sums(Xd, yd, self.coef_, self.intercept_, power=self.power)
+        return eng.tweedie_d2_from_sums(s, self.power)

@@ -11,8 +11,11 @@ Deliberate deviations (crash / hang fixes, documented in DESIGN.md):
   * Poisson: the reference fits and then raises AttributeError because it reads the
     pyglmnet attributes `beta_/beta0_` (backend/sglm.py:246-250); here `coef_/intercept_`
     are mapped, so Poisson fits are usable.
-  * Logistic / Multinomial / Gamma / general Tweedie are outside the hot-path scope
-    (SURVEY.md §8) and raise NotImplementedError.
+  * Gamma / Tweedie: the GPU path fits power 1 and any power > 1 with log link; power <= 0,
+    0 < power < 1 and link='identity' raise NotImplementedError.  With all-zero y and
+    1 < power < 2 the fit raises ValueError (scikit-learn returns an intercept of -inf).
+  * Logistic / Multinomial are outside the hot-path scope (SURVEY.md §8) and raise
+    NotImplementedError.
 """
 import time
 
@@ -99,7 +102,7 @@ class GLM():
         return -float(s[1] / s[0])
 
     def r2_score(self, X, y):
-        """model.score(X, y): R^2, or D^2 for the Poisson family (backend/sglm.py:169-184)."""
+        """model.score(X, y): R^2, or D^2 for the Poisson / Gamma / Tweedie families (backend/sglm.py:169-184)."""
         return self.model.score(X, y)
 
     # ------------------------------------------------------------------ fits

@@ -45,6 +45,13 @@ inline int sm_count() {
 template <typename T>
 __host__ __device__ inline T ceil_div(T a, T b) { return (a + b - 1) / b; }
 
+// Tweedie families with log link (the terms of scikit-learn's HalfTweedieLoss), a compile-time parameter of the GLM
+// passes: FAM_POISSON (power 1), FAM_GAMMA (power 2: Fisher weight 1), FAM_TWEEDIE (any other power > 1, a runtime
+// scalar; mu^(1-p) = exp((1-p) eta), one exp more per element).
+enum { FAM_POISSON = 0, FAM_GAMMA = 1, FAM_TWEEDIE = 2 };
+inline bool glm_power_ok(double power) { return power == 1.0 || power > 1.0; }
+inline int glm_family(double power) { return power == 1.0 ? FAM_POISSON : (power == 2.0 ? FAM_GAMMA : FAM_TWEEDIE); }
+
 // Soft-threshold branch select of the coordinate-descent step, (r > l1) ? dpos : ((r < -l1) ? dneg : other), as two
 // predicated selects.  Written in PTX because the compiler otherwise turns the nested conditional into a divergent
 // branch around the second FMA (BSSY / BRA / BSYNC + a BRA.DIV convergence check before the next shuffle) — on the

@@ -4,13 +4,14 @@
 // per loss / gradient evaluation — by one Newton-type iteration over the whole batch of B models:
 //
 //   eta  = X Wt + b          one fp64 GEMM  [T x C] x [C x B]: X is read ONCE per iteration for all B models
-//   R    = rw (mu - y)       fused elementwise epilogue + per-model sums (objective, sum mu, sum r), deterministic
+//   R    = rw dl/deta        fused elementwise epilogue + per-model sums (objective, sum of weights, sum R), deterministic;
+//                            templated on the family: Poisson rw (mu - y), Gamma rw (1 - y/mu), power p rw mu^(1-p) (mu - y)
 //   Gw   = X' R              one fp64 GEMM  [C x T] x [T x B] (split over T, partials added in fixed order)
 //   step                     per-model kernels: objective check / step halving, right-hand side H~ w - g, batched
 //                            triangular solves with the cached factor of (H~ + alpha n I), intercept, convergence
 //
-// H~ = X' diag(rw mu_ref) X is the weighted Gram of ONE reference model per fold (tcgen05 digit-plane Gram,
-// gram_tc.cu) shared by all alphas of the fold: exact gradient + approximate Hessian = the same fixed point as
+// H~ = X' diag(rw mu_ref^(2-p)) X (Fisher weights; Gamma: 1, so H~ = X' diag(rw) X for every iterate) is the weighted
+// Gram of ONE reference model per fold (tcgen05 digit-plane Gram, gram_tc.cu) shared by all alphas of the fold: exact gradient + approximate Hessian = the same fixed point as
 // Newton's iteration, reached at a linear rate; the host refreshes H~ when the steps stop contracting fast.
 // No host synchronisation inside an iteration (one small status read-back per iteration decides about refreshes).
 //
@@ -189,19 +190,26 @@ pb_reduce_splits_kernel(const double *__restrict__ part, long long n_elem, int n
 }
 
 // Elementwise pass over Eta [T][ldb] (thread <-> model column, CTA <-> row range): eta += b, mu = exp(eta).
-//   mode 0 (iteration): Eta <- rw (mu - y) in place; partial sums {rw (mu - y eta), rw mu, rw, rw (mu - y)}
+//   mode 0 (iteration): Eta <- R = rw dl/deta in place; partial sums {rw l, rw v, rw, R} with the loss l, its
+//                       derivative and the Fisher weight v of the family (HalfTweedieLoss, log link):
+//                         Poisson  l = mu - y eta                              dl/deta = mu - y            v = mu
+//                         Gamma    l = eta + y / mu                            dl/deta = 1 - y / mu        v = 1
+//                         power p  l = mu^(2-p)/(2-p) - y mu^(1-p)/(1-p)       dl/deta = mu^(1-p)(mu - y)  v = mu^(2-p)
 //   mode 1 (scores)   : no write; 2 x 8 sums per model for the row weights rw_a / rw_b (train / test):
-//                       {n, r^2, y, y^2, y eta, mu, y log y, r} with r = y - mu (as sglm_score_f64)
+//                       {n, r^2, y, y^2, s4, s5, s6, r} with r = y - mu; the family terms s4..s6 give the deviance:
+//                         Poisson {y eta, mu, y log y} (as sglm_score_f64), Gamma {eta, y / mu, log y},
+//                         power p {y mu^(1-p), mu^(2-p), y^(2-p)}
 // Y [T][ldy] holds the response columns (one per distinct `roll`), RW [n_w][ldrw] the row-weight vectors
 // (rw id < 0: all rows).  Partial sums per CTA -> pb_finish_sums_kernel adds them in fixed order.
 constexpr int PB_NS_IT = 4, PB_NS_SC = 16;
-template <int MODE>
+template <int MODE, int FAM>
 __global__ void __launch_bounds__(128)
 pb_epilogue_kernel(double *__restrict__ Eta, long long ldb, int n_models, long long T, const double *__restrict__ Y,
                    long long ldy, const int *__restrict__ ycol, const double *__restrict__ RW, long long ldrw,
                    const int *__restrict__ rw_a, const int *__restrict__ rw_b, const double *__restrict__ bvec,
-                   const int *__restrict__ status, double *__restrict__ partials) {
+                   const int *__restrict__ status, double power, double *__restrict__ partials) {
     constexpr int NS = MODE == 0 ? PB_NS_IT : PB_NS_SC;
+    const double q1 = 1.0 - power, inv1 = 1.0 / (1.0 - power), inv2 = 1.0 / (2.0 - power);   // FAM_TWEEDIE only
     const int mdl = blockIdx.y * 128 + threadIdx.x;
     const bool live = mdl < n_models;
     const long long rows_per = (T + gridDim.x - 1) / gridDim.x;
@@ -221,10 +229,22 @@ pb_epilogue_kernel(double *__restrict__ Eta, long long ldb, int n_models, long l
                 const double m = wa ? wa[t] : 1.0;
                 double r = 0.0;
                 if (m != 0.0) {
-                    const double mu = exp(eta);
-                    r = m * (mu - yt);
-                    acc[0] += m * (mu - yt * eta);
-                    acc[1] += m * mu;
+                    if (FAM == FAM_POISSON) {
+                        const double mu = exp(eta);
+                        r = m * (mu - yt);
+                        acc[0] += m * (mu - yt * eta);
+                        acc[1] += m * mu;
+                    } else if (FAM == FAM_GAMMA) {
+                        const double y_mu = yt * exp(-eta);
+                        r = m * (1.0 - y_mu);
+                        acc[0] += m * (eta + y_mu);
+                        acc[1] += m;
+                    } else {
+                        const double mu = exp(eta), mu1 = exp(q1 * eta), mu2 = mu * mu1;
+                        r = m * (mu1 * (mu - yt));
+                        acc[0] += m * (mu2 * inv2 - yt * mu1 * inv1);
+                        acc[1] += m * mu2;
+                    }
                     acc[2] += m;
                     acc[3] += r;
                 }
@@ -233,8 +253,16 @@ pb_epilogue_kernel(double *__restrict__ Eta, long long ldb, int n_models, long l
                 const double ma = wa ? wa[t] : 1.0, mb = (MODE == 1 && rw_b[mdl] < -1) ? 0.0 : (wb ? wb[t] : 1.0);
                 if (ma != 0.0 || mb != 0.0) {
                     const double mu = exp(eta), r = yt - mu;
-                    const double ylogy = (yt > 0.0) ? yt * log(yt) : 0.0;
-                    const double v[8] = {1.0, r * r, yt, yt * yt, yt * eta, mu, ylogy, r};
+                    double s4, s5, s6;
+                    if (FAM == FAM_POISSON) {
+                        s4 = yt * eta; s5 = mu; s6 = (yt > 0.0) ? yt * log(yt) : 0.0;
+                    } else if (FAM == FAM_GAMMA) {
+                        s4 = eta; s5 = yt / mu; s6 = log(yt);
+                    } else {
+                        const double mu1 = exp(q1 * eta);
+                        s4 = yt * mu1; s5 = mu * mu1; s6 = pow(yt, 2.0 - power);
+                    }
+                    const double v[8] = {1.0, r * r, yt, yt * yt, s4, s5, s6, r};
 #pragma unroll
                     for (int i = 0; i < 8; ++i) { acc[i] += ma * v[i]; acc[8 + i] += mb * v[i]; }
                 }
@@ -473,32 +501,68 @@ extern "C" size_t sglm_pb_epilogue_workspace_bytes(int64_t T, int32_t n_models) 
     return (size_t)pb_epi_grid(T) * (size_t)std::max(n_models, 1) * PB_NS_SC * sizeof(double);
 }
 
-// mode 0: Eta <- rw (mu - y) in place, sums [B][4]; mode 1: scores, sums [B][16]  (see pb_epilogue_kernel)
-extern "C" int sglm_pb_epilogue_f64(double *Eta, int64_t ldb, int32_t n_models, int64_t T, const double *Y,
-                                    int64_t ldy, const int32_t *ycol, const double *RW, int64_t ldrw,
-                                    const int32_t *rw_a, const int32_t *rw_b, const double *b,
-                                    const int32_t *status, int32_t mode, double *sums, void *workspace,
-                                    size_t workspace_bytes, void *stream) {
-    SGLM_CHECK_ARG(T >= 0 && n_models > 0 && ldb >= n_models && ldy >= 1, SGLM_E_SHAPE, "pb_epilogue: bad shape");
+template <int MODE>
+static void pb_epilogue_launch(int fam, dim3 grid, cudaStream_t st, double *Eta, int64_t ldb, int32_t n_models,
+                               int64_t T, const double *Y, int64_t ldy, const int32_t *ycol, const double *RW,
+                               int64_t ldrw, const int32_t *rw_a, const int32_t *rw_b, const double *b,
+                               const int32_t *status, double power, double *part) {
+    if (fam == FAM_POISSON)
+        pb_epilogue_kernel<MODE, FAM_POISSON><<<grid, 128, 0, st>>>(Eta, ldb, n_models, T, Y, ldy, ycol, RW, ldrw, rw_a,
+                                                                    rw_b, b, status, power, part);
+    else if (fam == FAM_GAMMA)
+        pb_epilogue_kernel<MODE, FAM_GAMMA><<<grid, 128, 0, st>>>(Eta, ldb, n_models, T, Y, ldy, ycol, RW, ldrw, rw_a,
+                                                                  rw_b, b, status, power, part);
+    else
+        pb_epilogue_kernel<MODE, FAM_TWEEDIE><<<grid, 128, 0, st>>>(Eta, ldb, n_models, T, Y, ldy, ycol, RW, ldrw, rw_a,
+                                                                    rw_b, b, status, power, part);
+}
+
+static int pb_epilogue(const char *name, double *Eta, int64_t ldb, int32_t n_models, int64_t T, const double *Y,
+                       int64_t ldy, const int32_t *ycol, const double *RW, int64_t ldrw, const int32_t *rw_a,
+                       const int32_t *rw_b, const double *b, const int32_t *status, double power, int32_t mode,
+                       double *sums, void *workspace, size_t workspace_bytes, void *stream) {
+    SGLM_CHECK_ARG(T >= 0 && n_models > 0 && ldb >= n_models && ldy >= 1, SGLM_E_SHAPE, "%s: bad shape", name);
     SGLM_CHECK_ARG(Eta && Y && ycol && rw_a && b && sums && workspace && (mode == 0 || rw_b), SGLM_E_INVALID_ARG,
-                   "pb_epilogue: null pointer");
+                   "%s: null pointer", name);
+    SGLM_CHECK_ARG(glm_power_ok(power), SGLM_E_UNSUPPORTED, "%s: power %g (supported: 1 and > 1, log link)", name, power);
     SGLM_CHECK_ARG(workspace_bytes >= sglm_pb_epilogue_workspace_bytes(T, n_models), SGLM_E_WORKSPACE,
-                   "pb_epilogue: workspace too small");
+                   "%s: workspace too small", name);
     cudaStream_t st = (cudaStream_t)stream;
     const int gx = pb_epi_grid(T);
     dim3 grid((unsigned)gx, (unsigned)ceil_div(n_models, 128));
     const int NS = mode == 0 ? PB_NS_IT : PB_NS_SC;
+    const int fam = glm_family(power);
     if (mode == 0)
-        pb_epilogue_kernel<0><<<grid, 128, 0, st>>>(Eta, ldb, n_models, T, Y, ldy, ycol, RW, ldrw, rw_a, rw_b, b, status,
-                                                    (double *)workspace);
+        pb_epilogue_launch<0>(fam, grid, st, Eta, ldb, n_models, T, Y, ldy, ycol, RW, ldrw, rw_a, rw_b, b, status, power,
+                              (double *)workspace);
     else
-        pb_epilogue_kernel<1><<<grid, 128, 0, st>>>(Eta, ldb, n_models, T, Y, ldy, ycol, RW, ldrw, rw_a, rw_b, b, status,
-                                                    (double *)workspace);
+        pb_epilogue_launch<1>(fam, grid, st, Eta, ldb, n_models, T, Y, ldy, ycol, RW, ldrw, rw_a, rw_b, b, status, power,
+                              (double *)workspace);
     SGLM_LAUNCH_OK("pb_epilogue_kernel");
     const long long n_vals = (long long)n_models * NS;
     pb_finish_sums_kernel<<<(unsigned)ceil_div<long long>(n_vals, 256), 256, 0, st>>>((const double *)workspace, gx, n_vals, sums);
     SGLM_LAUNCH_OK("pb_finish_sums_kernel");
     return SGLM_OK;
+}
+
+// Poisson: mode 0: Eta <- rw (mu - y) in place, sums [B][4]; mode 1: scores, sums [B][16]  (see pb_epilogue_kernel)
+extern "C" int sglm_pb_epilogue_f64(double *Eta, int64_t ldb, int32_t n_models, int64_t T, const double *Y,
+                                    int64_t ldy, const int32_t *ycol, const double *RW, int64_t ldrw,
+                                    const int32_t *rw_a, const int32_t *rw_b, const double *b,
+                                    const int32_t *status, int32_t mode, double *sums, void *workspace,
+                                    size_t workspace_bytes, void *stream) {
+    return pb_epilogue("pb_epilogue", Eta, ldb, n_models, T, Y, ldy, ycol, RW, ldrw, rw_a, rw_b, b, status, 1.0, mode,
+                       sums, workspace, workspace_bytes, stream);
+}
+
+// The same for the Tweedie family of `power` (1, or > 1; log link)
+extern "C" int sglm_glm_epilogue_f64(double *Eta, int64_t ldb, int32_t n_models, int64_t T, const double *Y,
+                                     int64_t ldy, const int32_t *ycol, const double *RW, int64_t ldrw,
+                                     const int32_t *rw_a, const int32_t *rw_b, const double *b,
+                                     const int32_t *status, double power, int32_t mode, double *sums, void *workspace,
+                                     size_t workspace_bytes, void *stream) {
+    return pb_epilogue("glm_epilogue", Eta, ldb, n_models, T, Y, ldy, ycol, RW, ldrw, rw_a, rw_b, b, status, power, mode,
+                       sums, workspace, workspace_bytes, stream);
 }
 
 // One chord step of every active model: objective check / halving + right-hand sides, batched triangular solves with

@@ -1,4 +1,4 @@
-// Explicit-matrix passes: predict, fused residual/score sums, Poisson IRLS preparation.
+// Explicit-matrix passes: predict, fused residual/score sums, IRLS preparation (Poisson, Gamma, Tweedie power > 1).
 // Replaces GLM.predict / neg_mse_score / r2_score / get_residuals (reference
 // backend/sglm.py:150-184, :314-347) and one evaluation of the TweedieRegressor(power=1)
 // loss/gradient/Hessian weights (sklearn/linear_model/_glm/glm.py:276-316).
@@ -40,11 +40,12 @@ __device__ __forceinline__ double row_dot(const double *__restrict__ row, const 
     return warp_sum(s);
 }
 
-template <int MODE>
+// MODE_SCORE / MODE_IRLS: FAM selects the family terms (common.cuh); the power is read by FAM_TWEEDIE only
+template <int MODE, int FAM = FAM_POISSON>
 __global__ void __launch_bounds__(PR_THREADS)
 row_pass_kernel(const double *__restrict__ X, long long ldx, const double *__restrict__ y,
                 const double *__restrict__ rw, long long T, int C, const double *__restrict__ w,
-                const double *__restrict__ b_dev, int link, double *__restrict__ out0,
+                const double *__restrict__ b_dev, int link, double power, double *__restrict__ out0,
                 double *__restrict__ out1, double *__restrict__ partials) {
     extern __shared__ __align__(16) double ws[];
     for (int j = threadIdx.x; j < C; j += PR_THREADS) ws[j] = w[j];
@@ -72,9 +73,20 @@ row_pass_kernel(const double *__restrict__ X, long long ldx, const double *__res
                     acc[1] += m * r * r;
                     acc[2] += m * yt;
                     acc[3] += m * yt * yt;
-                    acc[4] += m * yt * eta;
-                    acc[5] += m * mu;
-                    acc[6] += (yt > 0.0) ? m * yt * log(yt) : 0.0;
+                    if (FAM == FAM_POISSON) {
+                        acc[4] += m * yt * eta;
+                        acc[5] += m * mu;
+                        acc[6] += (yt > 0.0) ? m * yt * log(yt) : 0.0;
+                    } else if (FAM == FAM_GAMMA) {             // deviance terms, see pb_epilogue_kernel
+                        acc[4] += m * eta;
+                        acc[5] += m * (yt / mu);
+                        acc[6] += m * log(yt);
+                    } else {
+                        const double mu1 = exp((1.0 - power) * eta);
+                        acc[4] += m * (yt * mu1);
+                        acc[5] += m * (mu * mu1);
+                        acc[6] += m * pow(yt, 2.0 - power);
+                    }
                     acc[7] += m * r;
                 }
             } else {
@@ -82,10 +94,21 @@ row_pass_kernel(const double *__restrict__ X, long long ldx, const double *__res
                 if (m != 0.0) {
                     const double mu = exp(eta);
                     const double yt = y[t];
-                    out0[t] = m * mu;                       // IRLS weight
+                    if (FAM == FAM_POISSON) {
+                        out0[t] = m * mu;                   // IRLS weight
+                        acc[0] += m * (mu - yt * eta);
+                        acc[1] += m * mu;
+                    } else if (FAM == FAM_GAMMA) {
+                        out0[t] = m;                        // Fisher weight mu^(2-p) = 1
+                        acc[0] += m * (eta + yt / mu);
+                        acc[1] += m;
+                    } else {
+                        const double mu1 = exp((1.0 - power) * eta), mu2 = mu * mu1;
+                        out0[t] = m * mu2;
+                        acc[0] += m * (mu2 / (2.0 - power) - yt * mu1 / (1.0 - power));
+                        acc[1] += m * mu2;
+                    }
                     out1[t] = eta + (yt - mu) / mu;         // working response
-                    acc[0] += m * (mu - yt * eta);
-                    acc[1] += m * mu;
                     acc[2] += m;
                     acc[3] += m * yt;
                 } else {                                    // row not in this fold
@@ -184,9 +207,40 @@ extern "C" int sglm_predict_f64(const double *X, int64_t ldx, int64_t T, int32_t
     SGLM_CHECK_ARG(smem <= 200 * 1024, SGLM_E_UNSUPPORTED, "predict: C=%d too large", C);
     SGLM_CUDA_OK(cudaFuncSetAttribute(row_pass_kernel<MODE_PREDICT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     row_pass_kernel<MODE_PREDICT><<<pass_grid(T), PR_THREADS, smem, (cudaStream_t)stream>>>(
-        X, ldx, nullptr, nullptr, T, C, w, b_dev, link, out, nullptr, nullptr);
+        X, ldx, nullptr, nullptr, T, C, w, b_dev, link, 1.0, out, nullptr, nullptr);
     SGLM_LAUNCH_OK("row_pass_kernel<predict>");
     return SGLM_OK;
+}
+
+// one fused pass (MODE_SCORE or MODE_IRLS) of the family of `power` + the fixed-order reduction of its sums
+template <int MODE, int FAM>
+static int row_pass_sums(const double *X, int64_t ldx, const double *y, const double *rw, int64_t T, int32_t C,
+                         const double *w, const double *b_dev, int32_t link, double power, double *out0, double *out1,
+                         double *sums, void *workspace, void *stream) {
+    const size_t smem = (size_t)((C + 1) & ~1) * sizeof(double);
+    const int grid = pass_grid(T);
+    cudaStream_t st = (cudaStream_t)stream;
+    SGLM_CUDA_OK(cudaFuncSetAttribute(row_pass_kernel<MODE, FAM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    row_pass_kernel<MODE, FAM><<<grid, PR_THREADS, smem, st>>>(X, ldx, y, rw, T, C, w, b_dev, link, power, out0, out1,
+                                                               (double *)workspace);
+    SGLM_LAUNCH_OK(MODE == MODE_SCORE ? "row_pass_kernel<score>" : "row_pass_kernel<irls>");
+    finish_sums_kernel<<<1, 256, 0, st>>>((const double *)workspace, grid, sums);
+    SGLM_LAUNCH_OK("finish_sums_kernel");
+    return SGLM_OK;
+}
+
+template <int MODE>
+static int row_pass_sums_family(const double *X, int64_t ldx, const double *y, const double *rw, int64_t T, int32_t C,
+                                const double *w, const double *b_dev, int32_t link, double power, double *out0,
+                                double *out1, double *sums, void *workspace, void *stream) {
+    switch (glm_family(power)) {
+    case FAM_POISSON:
+        return row_pass_sums<MODE, FAM_POISSON>(X, ldx, y, rw, T, C, w, b_dev, link, power, out0, out1, sums, workspace, stream);
+    case FAM_GAMMA:
+        return row_pass_sums<MODE, FAM_GAMMA>(X, ldx, y, rw, T, C, w, b_dev, link, power, out0, out1, sums, workspace, stream);
+    default:
+        return row_pass_sums<MODE, FAM_TWEEDIE>(X, ldx, y, rw, T, C, w, b_dev, link, power, out0, out1, sums, workspace, stream);
+    }
 }
 
 extern "C" int sglm_score_f64(const double *X, int64_t ldx, const double *y, const double *rw, int64_t T,
@@ -194,17 +248,20 @@ extern "C" int sglm_score_f64(const double *X, int64_t ldx, const double *y, con
                               double *sums, void *workspace, void *stream) {
     SGLM_CHECK_ARG(T >= 0 && C > 0 && ldx >= C, SGLM_E_SHAPE, "score: bad shape");
     SGLM_CHECK_ARG(X && y && w && sums && workspace, SGLM_E_INVALID_ARG, "score: null pointer");
-    const size_t smem = (size_t)((C + 1) & ~1) * sizeof(double);
-    SGLM_CHECK_ARG(smem <= 200 * 1024, SGLM_E_UNSUPPORTED, "score: C=%d too large", C);
-    const int grid = pass_grid(T);
-    cudaStream_t st = (cudaStream_t)stream;
-    SGLM_CUDA_OK(cudaFuncSetAttribute(row_pass_kernel<MODE_SCORE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    row_pass_kernel<MODE_SCORE><<<grid, PR_THREADS, smem, st>>>(X, ldx, y, rw, T, C, w, b_dev, link, resid,
-                                                                nullptr, (double *)workspace);
-    SGLM_LAUNCH_OK("row_pass_kernel<score>");
-    finish_sums_kernel<<<1, 256, 0, st>>>((const double *)workspace, grid, sums);
-    SGLM_LAUNCH_OK("finish_sums_kernel");
-    return SGLM_OK;
+    SGLM_CHECK_ARG((size_t)((C + 1) & ~1) * sizeof(double) <= 200 * 1024, SGLM_E_UNSUPPORTED, "score: C=%d too large", C);
+    return row_pass_sums<MODE_SCORE, FAM_POISSON>(X, ldx, y, rw, T, C, w, b_dev, link, 1.0, resid, nullptr, sums,
+                                                  workspace, stream);
+}
+
+extern "C" int sglm_score_glm_f64(const double *X, int64_t ldx, const double *y, const double *rw, int64_t T,
+                                  int32_t C, const double *w, const double *b_dev, double power, double *resid,
+                                  double *sums, void *workspace, void *stream) {
+    SGLM_CHECK_ARG(T >= 0 && C > 0 && ldx >= C, SGLM_E_SHAPE, "score_glm: bad shape");
+    SGLM_CHECK_ARG(X && y && w && sums && workspace, SGLM_E_INVALID_ARG, "score_glm: null pointer");
+    SGLM_CHECK_ARG(glm_power_ok(power), SGLM_E_UNSUPPORTED, "score_glm: power %g (supported: 1 and > 1, log link)", power);
+    SGLM_CHECK_ARG((size_t)((C + 1) & ~1) * sizeof(double) <= 200 * 1024, SGLM_E_UNSUPPORTED, "score_glm: C=%d too large", C);
+    return row_pass_sums_family<MODE_SCORE>(X, ldx, y, rw, T, C, w, b_dev, 1, power, resid, nullptr, sums, workspace,
+                                            stream);
 }
 
 extern "C" int sglm_poisson_irls_prepare_f64(const double *X, int64_t ldx, const double *y, const double *rw,
@@ -213,17 +270,21 @@ extern "C" int sglm_poisson_irls_prepare_f64(const double *X, int64_t ldx, const
                                              void *stream) {
     SGLM_CHECK_ARG(T >= 0 && C > 0 && ldx >= C, SGLM_E_SHAPE, "irls_prepare: bad shape");
     SGLM_CHECK_ARG(X && y && w && weight && z && sums && workspace, SGLM_E_INVALID_ARG, "irls_prepare: null pointer");
-    const size_t smem = (size_t)((C + 1) & ~1) * sizeof(double);
-    SGLM_CHECK_ARG(smem <= 200 * 1024, SGLM_E_UNSUPPORTED, "irls_prepare: C=%d too large", C);
-    const int grid = pass_grid(T);
-    cudaStream_t st = (cudaStream_t)stream;
-    SGLM_CUDA_OK(cudaFuncSetAttribute(row_pass_kernel<MODE_IRLS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    row_pass_kernel<MODE_IRLS><<<grid, PR_THREADS, smem, st>>>(X, ldx, y, rw, T, C, w, b_dev, 1, weight, z,
-                                                               (double *)workspace);
-    SGLM_LAUNCH_OK("row_pass_kernel<irls>");
-    finish_sums_kernel<<<1, 256, 0, st>>>((const double *)workspace, grid, sums);
-    SGLM_LAUNCH_OK("finish_sums_kernel");
-    return SGLM_OK;
+    SGLM_CHECK_ARG((size_t)((C + 1) & ~1) * sizeof(double) <= 200 * 1024, SGLM_E_UNSUPPORTED, "irls_prepare: C=%d too large", C);
+    return row_pass_sums<MODE_IRLS, FAM_POISSON>(X, ldx, y, rw, T, C, w, b_dev, 1, 1.0, weight, z, sums, workspace,
+                                                 stream);
+}
+
+extern "C" int sglm_glm_irls_prepare_f64(const double *X, int64_t ldx, const double *y, const double *rw,
+                                         int64_t T, int32_t C, const double *w, const double *b_dev, double power,
+                                         double *weight, double *z, double *sums, void *workspace, void *stream) {
+    SGLM_CHECK_ARG(T >= 0 && C > 0 && ldx >= C, SGLM_E_SHAPE, "glm_irls_prepare: bad shape");
+    SGLM_CHECK_ARG(X && y && w && weight && z && sums && workspace, SGLM_E_INVALID_ARG, "glm_irls_prepare: null pointer");
+    SGLM_CHECK_ARG(glm_power_ok(power), SGLM_E_UNSUPPORTED, "glm_irls_prepare: power %g (supported: 1 and > 1, log link)",
+                   power);
+    SGLM_CHECK_ARG((size_t)((C + 1) & ~1) * sizeof(double) <= 200 * 1024, SGLM_E_UNSUPPORTED,
+                   "glm_irls_prepare: C=%d too large", C);
+    return row_pass_sums_family<MODE_IRLS>(X, ldx, y, rw, T, C, w, b_dev, 1, power, weight, z, sums, workspace, stream);
 }
 
 extern "C" size_t sglm_xt_vec_workspace_bytes(int32_t C) { return (size_t)sm_count() * 8 * (size_t)std::max(C, 1) * sizeof(double); }

@@ -494,11 +494,13 @@ def _set_fitted(glm, coef, intercept, info, status):
     glm.beta0_ = glm.intercept_
 
 
-def _poisson_grid(Xd, yd, cv_idx, glms, rolls, score_method):
-    """Poisson family (backend/sglm.py:112-115): every (parameter set, fold) fit and every refit of the grid as ONE
-    batched Newton-type iteration (`_engine.poisson_grid_batched`: X is read once per iteration for all models,
-    one tcgen05 weighted Gram per fold as the shared approximate Hessian, exact gradients), then one batched
-    scoring pass for the train / test sums of every fold model."""
+def _poisson_grid(Xd, yd, cv_idx, glms, rolls, score_method, power=1.0):
+    """Poisson family (backend/sglm.py:112-115), or the Tweedie family of `power` > 1 (Gamma: power 2, :112-117):
+    every (parameter set, fold) fit and every refit of the grid as ONE batched Newton-type iteration
+    (`_engine.tweedie_grid_batched`: X is read once per iteration for all models, one tcgen05 weighted Gram per fold
+    as the shared approximate Hessian, exact gradients), then one batched scoring pass for the train / test sums of
+    every fold model.  'r2' scores are the family's D^2; -MSE and the pooled cv_R2_score / cv_mse_score are
+    residual-based."""
     import torch
     T, C = Xd.shape
     F = len(cv_idx)
@@ -523,8 +525,8 @@ def _poisson_grid(Xd, yd, cv_idx, glms, rolls, score_method):
             ycol.append(ycol_of_roll[r]); rw_a.append(f); rw_b.append(F + f)
         models.append(eng.PoissonModel(est.alpha, est.fit_intercept, rw=-1, ycol=0, max_iter=est.max_iter, tol=est.tol))
         ycol.append(0); rw_a.append(-1); rw_b.append(-2)          # the refit uses the UN-rolled y (backend/sglm_cv.py:181)
-    Wd, bd, n_it, status = eng.poisson_grid_batched(Xd, Yd, models, RW)
-    sums = eng.poisson_scores_batched(Xd, Yd, Wd, bd, ycol, rw_a, rw_b, RW)
+    Wd, bd, n_it, status = eng.tweedie_grid_batched(Xd, Yd, models, RW, power)
+    sums = eng.tweedie_scores_batched(Xd, Yd, Wd, bd, ycol, rw_a, rw_b, RW, power)
     W_h, b_h = Wd.cpu().numpy(), bd.cpu().numpy()
     results = []
     for k, glm in enumerate(glms):
@@ -537,7 +539,7 @@ def _poisson_grid(Xd, yd, cv_idx, glms, rolls, score_method):
         for f in range(F):
             st, se = sums[base + f, 0], sums[base + f, 1]
             if score_method == 'r2':
-                s_tr[f], s_te[f] = eng.poisson_d2_from_sums(st), eng.poisson_d2_from_sums(se)
+                s_tr[f], s_te[f] = eng.tweedie_d2_from_sums(st, power), eng.tweedie_d2_from_sums(se, power)
             else:
                 s_tr[f], s_te[f] = -st[1] / st[0], -se[1] / se[0]
             rss_pool += se[1]
@@ -573,16 +575,20 @@ def _cv_batch(X, y, cv_idx, entries, beta_, beta0_, score_method):
         glms.append(sglm_.GLM(model_name, beta0_=beta0_, beta_=beta_, **kw))   # refit object (:180)
     out = [None] * len(entries)
     gauss = [i for i, g in enumerate(glms) if g.model.kind in ("ols", "ridge", "lasso", "enet")]
-    pois = [i for i, g in enumerate(glms) if g.model.kind == "poisson"]
+    # the log-link families: one batch per distinct power, Poisson (power 1) first
+    by_power = {}
+    for i, g in enumerate(glms):
+        if g.model.kind in ("poisson", "tweedie"):
+            by_power.setdefault(1.0 if g.model.kind == "poisson" else g.model.power, []).append(i)
     if gauss:
         res = _gaussian_grid(Xd, yd, cv_idx, [glms[i] for i in gauss], [rolls[i] for i in gauss], score_method)
         for i, r in zip(gauss, res):
             out[i] = r
-    if pois:
-        if isinstance(Xd, eng.LagRecipe):
-            Xd = Xd.tensor()
-        res = _poisson_grid(Xd, yd, cv_idx, [glms[i] for i in pois], [rolls[i] for i in pois], score_method)
-        for i, r in zip(pois, res):
+    if by_power and isinstance(Xd, eng.LagRecipe):
+        Xd = Xd.tensor()
+    for power, idx in by_power.items():
+        res = _poisson_grid(Xd, yd, cv_idx, [glms[i] for i in idx], [rolls[i] for i in idx], score_method, power)
+        for i, r in zip(idx, res):
             out[i] = r
     for (model_name, kw), r in zip(entries, out):
         r['glm_kwargs'] = kw

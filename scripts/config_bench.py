@@ -1,10 +1,11 @@
 """The other BASELINE.json configurations on one B200, each with the reference's CPU path timed beside it
 (SURVEY.md §8d): configs[0] single ElasticNet fit 100k x 410, configs[1] Ridge CV 5 folds x 20 alphas 500k x 1220,
-configs[3] Poisson alpha sweep 20 alphas x 5 folds (+ refits) 1M x 800.  One JSON line per configuration:
+configs[3] Poisson alpha sweep 20 alphas x 5 folds (+ refits) 1M x 800, and the same sweep for the Gamma family (c4g)
+and the Tweedie family with power 1.5 (c4t) on a response of that family.  One JSON line per configuration:
 device-resident time (CUDA events, warm-up excluded), end-to-end time from host numpy arrays, per-entry-point
 milliseconds, and the CPU baseline (scikit-learn through the oracle port, bounded sample, extrapolated and labelled).
 
-    python scripts/config_bench.py [c1] [c2] [c4] [--no-cpu]
+    python scripts/config_bench.py [c1] [c2] [c4] [c4g] [c4t] [--no-cpu]     (default: c1 c2 c4)
 """
 import json
 import os
@@ -29,7 +30,7 @@ warnings.filterwarnings("ignore")
 CORES = len(os.sched_getaffinity(0))
 
 
-def session(T, P, lo, hi, seed, poisson=False):
+def session(T, P, lo, hi, seed, poisson=False, power=None):
     shifts = [0] + [s for s in range(lo, hi + 1) if s != 0]
     X0_h = synth_data.synth_base(T, P, seed)
     X0 = torch.from_numpy(X0_h).cuda()
@@ -41,6 +42,10 @@ def session(T, P, lo, hi, seed, poisson=False):
     if poisson:
         z = (s - s.mean()) / s.std()
         y = torch.poisson(torch.exp(0.3 * z - 1.0))
+    elif power is not None:
+        z = (s - s.mean()) / s.std()
+        mu = torch.exp(0.3 * z - 1.0).cpu().numpy()
+        y = torch.from_numpy(synth_data.tweedie_draw(mu, seed, power)).cuda()
     else:
         y = s + 1.5 * s.std() * torch.randn_like(s)
         y = (y - y.mean()) / y.std()
@@ -191,10 +196,36 @@ def run_c4(cpu):
     return line
 
 
+def run_c4_family(name, model_name, power):
+    """c4 with the response and the family of `model_name` (log link): the same design, folds and alpha sweep."""
+    X0_h, X0, shifts, (lo, hi), y, n = session(1_000_000, 20, -20, 19, 4, power=power)
+    folds_h = synth_data.synth_folds(n, 5, 4)
+    folds = [(torch.from_numpy(a).cuda(), torch.from_numpy(b).cuda()) for a, b in folds_h]
+    extra = {} if model_name == "Gamma" else {"power": power}
+    grid = [dict(alpha=float(a), model_name=model_name, **extra) for a in np.logspace(-4, 1, 20)]
+
+    def dev():
+        d = sglm_pp.timeshift_multiple(X0, shift_amt_list=shifts)[lo:hi]
+        return sglm_cv.cv_glm_mult_params(d, y, folds, model_name, [dict(g) for g in grid], score_method="r2")
+    sec, r, per = timed(dev, reps=2, warm=1)
+    diag = _engine.last_poisson_batch
+    return {"config": "%s: %s GLM (power %g, log link, L2) alpha sweep logspace(-4, 1, 20) x (5 folds + refit) = 120 fits, "
+                      "1M timepoints x 20 predictors x 40 shifts = 800 columns, response of the family, every fit driven to "
+                      "its optimum (step bound 1e-8)" % (name, model_name, power),
+            "fits": 120, "seconds": sec, "fits_per_s": 120 / sec, "best_params": r["best_params"], "batch": diag,
+            "rounds": diag[0]["rounds"] if diag else None,
+            "refreshes": diag[0]["refreshes"] if diag else None,
+            "n_iter_min_max": [int(min(np.min(x["_fit_info"]["n_iter"]) for x in r["full_cv_results"])),
+                               int(max(np.max(x["_fit_info"]["n_iter"]) for x in r["full_cv_results"]))],
+            "per_entry_ms": per}
+
+
 if __name__ == "__main__":
     which = [a for a in sys.argv[1:] if not a.startswith("--")] or ["c1", "c2", "c4"]
     cpu = "--no-cpu" not in sys.argv
+    runs = {"c1": run_c1, "c2": run_c2, "c4": run_c4,
+            "c4g": lambda cpu: run_c4_family("c4g", "Gamma", 2.0), "c4t": lambda cpu: run_c4_family("c4t", "Tweedie", 1.5)}
     for name in which:
-        line = {"c1": run_c1, "c2": run_c2, "c4": run_c4}[name](cpu)
+        line = runs[name](cpu)
         print(json.dumps(line), flush=True)
         torch.cuda.empty_cache()

@@ -3,8 +3,8 @@ Seeded synthetic "photometry-shaped" inputs (SURVEY.md §8d) shared by tests, th
 bench.py.  Neutral utility: neither product code nor oracle.  Shapes follow the reference's
 drivers: sparse 0/1 event indicators (er_refactored_from_scratch_cleanup.py:203-222), a few
 real-valued z-scored AR(1) signals and one within-trial ramp (pp_design_mat.py:171); smooth
-exponentially decaying kernels; Gaussian response with AR(1) noise scaled to R^2 ~ 0.3 or a
-spike-count-like Poisson response; GroupShuffleSplit-style folds over 1000-row trials
+exponentially decaying kernels; Gaussian response with AR(1) noise scaled to R^2 ~ 0.3, a
+spike-count-like Poisson response, or a Gamma / compound Poisson-Gamma / inverse Gaussian one; GroupShuffleSplit-style folds over 1000-row trials
 (backend/sglm_pp.py:262-263).
 """
 import numpy as np
@@ -50,6 +50,34 @@ def synth_response(Xd, beta, seed, poisson=False):
     e = e / e.std() * s.std() * np.sqrt(0.7 / 0.3)
     y = s + e
     return (y - y.mean()) / y.std()
+
+
+def synth_response_tweedie(Xd, beta, seed, power):
+    """Response of the Tweedie family of `power` with log link and mean mu = exp(0.3 z(X beta) - 1), as the
+    Poisson response: power 2 Gamma (shape 2), 1 < power < 2 compound Poisson-Gamma with dispersion 1 (exact
+    zeros), power 3 inverse Gaussian (numpy Wald, dispersion 1)."""
+    s = Xd @ beta
+    z = (s - s.mean()) / (s.std() + 1e-300)
+    return tweedie_draw(np.exp(0.3 * z - 1.0), seed, power)
+
+
+def tweedie_draw(mu, seed, power):
+    """One draw per mean mu of the distributions of synth_response_tweedie."""
+    rng = np.random.default_rng(seed + 17)
+    mu = np.asarray(mu, dtype=np.float64)
+    if power == 2:
+        return rng.gamma(2.0, mu / 2.0)
+    if power == 3:
+        return rng.wald(mu, 1.0)
+    if 1 < power < 2:
+        # N ~ Poisson(mu^(2-p) / (2-p)) events, each Gamma(shape (2-p)/(p-1), scale (p-1) mu^(p-1))
+        n = rng.poisson(mu ** (2.0 - power) / (2.0 - power))
+        shape = n * (2.0 - power) / (power - 1.0)
+        y = np.zeros_like(mu)
+        pos = n > 0
+        y[pos] = rng.gamma(shape[pos], (power - 1.0) * mu[pos] ** (power - 1.0))
+        return y
+    raise ValueError(f"no synthetic Tweedie response for power={power} (1 < power < 2, 2 or 3)")
 
 
 def synth_folds(T, n_folds, seed, group=1000, test_size=0.2):
