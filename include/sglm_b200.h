@@ -205,6 +205,20 @@ int sglm_gram_tc_cells_partial_f64(const double *X, int64_t ldx, const double *Y
                                    int32_t C, const int32_t *colE, const int32_t *colS, const int32_t *colS_host,
                                    int32_t n_cells, const int64_t *cell_rows_host, const int64_t *rows, int32_t n_out,
                                    const int32_t *member_host, void *workspace, size_t workspace_bytes, void *stream);
+/* Row-sharded WEIGHTED Gram (the Hessian X' diag(w) X of a row-sharded GLM iteration), rows of Z scaled by row_scale:
+ *   colstats_scaled : sglm_gram_tc_colstats_f64 with row_scale (NULL only when T == 0); the ranks combine (max / min),
+ *                     then sglm_gram_tc_exponents with the Gram's max_planes;
+ *   scaled_partial  : sglm_gram_tc_cells_partial_f64 with row_scale; finish with sglm_gram_tc_cells_combine_f64.
+ * The int64 partials summed over ANY partition of the rows, then combined, are the bits of sglm_gram_tc_scaled_f64
+ * over all rows. */
+int sglm_gram_tc_colstats_scaled_f64(const double *X, int64_t ldx, const double *Y, int64_t ldy, int32_t n_y, int64_t T,
+                                     int32_t C, const double *row_scale, uint64_t *colmax_bits, int32_t *col_lsb,
+                                     void *stream);
+int sglm_gram_tc_scaled_partial_f64(const double *X, int64_t ldx, const double *Y, int64_t ldy, int32_t n_y, int64_t T,
+                                    int32_t C, const double *row_scale, const int32_t *colE, const int32_t *colS,
+                                    const int32_t *colS_host, int32_t n_cells, const int64_t *cell_rows_host,
+                                    const int64_t *rows, int32_t n_out, const int32_t *member_host, void *workspace,
+                                    size_t workspace_bytes, void *stream);
 int sglm_gram_tc_cells_combine_f64(int32_t C, int32_t n_y, const int32_t *colE, const int32_t *colS,
                                    const int32_t *colS_host, int32_t n_cells, const int64_t *cell_rows_host,
                                    int32_t n_out, double *G, int64_t ldg, void *workspace, size_t workspace_bytes,
@@ -472,6 +486,9 @@ int sglm_glm_epilogue_f64(double *Eta, int64_t ldb, int32_t n_models, int64_t T,
                           const int32_t *ycol, const double *RW, int64_t ldrw, const int32_t *rw_a,
                           const int32_t *rw_b, const double *b, const int32_t *status, double power, int32_t mode,
                           double *sums, void *workspace, size_t workspace_bytes, void *stream);
+/* out[e] = parts[0][e] + parts[1][e] + ... in that order (parts [n_parts][n_elem]): the fixed-order sum of per-rank
+ * fp64 partials gathered in rank order, so every rank of a row-sharded batch holds the same bits. */
+int sglm_reduce_parts_f64(const double *parts, int64_t n_elem, int32_t n_parts, double *out, void *stream);
 int sglm_pb_state_words(void);
 int sglm_pb_step_f64(const uint64_t *state_host, const double *const *L_of, void *stream);
 

@@ -161,7 +161,14 @@ class LagRecipe:
 
     def tensor(self):
         if self._cache is None:
-            self._cache = gather(self.base, self.src, self.sh, self.fill)[self.lo:self.hi]
+            # only the base rows the range reads (lag halo included): a row slice of a long session (one rank of a
+            # row-sharded grid) costs its own rows, not the whole session
+            sh_max, sh_min = (int(self.sh.max()), int(self.sh.min())) if self.sh.size else (0, 0)
+            a = max(0, min(self.lo, self.lo - sh_max))
+            b = min(int(self.base.shape[0]), max(self.hi, self.hi - sh_min))
+            if b <= a:
+                a = b = min(max(self.lo, 0), int(self.base.shape[0]))
+            self._cache = gather(self.base[a:b], self.src, self.sh, self.fill)[self.lo - a:self.hi - a]
         return self._cache
 
 
@@ -1114,6 +1121,61 @@ def suffstats_tc_scaled(Xd, Yd, rs, max_planes, rows=None):
     return G
 
 
+def suffstats_tc_scaled_sharded(Xd, Yd, rs, max_planes, all_reduce):
+    """suffstats_tc_scaled when this process holds a SLICE of the rows (all_reduce as in suffstats_tc_sharded): the
+    column analysis is combined over the processes (max / min), every process slices its rows and the int64 plane
+    Grams are summed (exact), so G has the bits of the one-GPU weighted Gram over all rows, on every process."""
+    torch = nat.require_cuda()
+    T, C = Xd.shape
+    n_y = Yd.shape[1]
+    n_aug = C + n_y + 1
+    ldg = _round_up(n_aug, 8)
+    colmax = torch.empty(n_aug, dtype=torch.int64, device="cuda")
+    colS = torch.empty(n_aug, dtype=torch.int32, device="cuda")
+    colE = torch.empty(n_aug, dtype=torch.int32, device="cuda")
+    flag = torch.empty(1, dtype=torch.int32, device="cuda")
+    call("sglm_gram_tc_colstats_scaled_f64", ptr(Xd), row_stride(Xd), ptr(Yd), row_stride(Yd), n_y, T, C, ptr(rs),
+         ptr(colmax), ptr(colS), stream_ptr())
+    all_reduce(colmax, "max")
+    all_reduce(colS, "min")
+    call("sglm_gram_tc_exponents", ptr(colmax), n_aug, int(max_planes), ptr(colE), ptr(colS), ptr(flag), stream_ptr())
+    host = torch.cat([colS, flag]).cpu().numpy()
+    if host[-1] != 0:
+        raise ValueError("Input contains NaN, infinity or a value too large for dtype('float64').")
+    colS_h = np.ascontiguousarray(host[:-1], dtype=np.int32)
+    rows = torch.full((max(_round_up(T, 128), 128),), -1, dtype=torch.int64, device="cuda")
+    rows[:T] = torch.arange(T, dtype=torch.int64, device="cuda")
+    sizes = np.ascontiguousarray([T], dtype=np.int64)
+    member = np.ones((1, 1), dtype=np.int32)
+    colS_p, sizes_p = colS_h.ctypes.data_as(ctypes.c_void_p), sizes.ctypes.data_as(ctypes.c_void_p)
+    ws_bytes = nat.lib().sglm_gram_tc_cells_workspace_bytes(n_aug, colS_p, 1, sizes_p, 1)
+    if ws_bytes == 0:
+        raise nat.SglmNativeError("gram_tc: invalid plan")
+    off_b, size_b = ctypes.c_uint64(0), ctypes.c_uint64(0)
+    if nat.lib().sglm_gram_tc_cells_sgout(n_aug, colS_p, 1, sizes_p, 1, ctypes.byref(off_b), ctypes.byref(size_b)) != 0:
+        raise nat.SglmNativeError("gram_tc: " + nat.lib().sglm_last_error().decode())
+    raw = torch.empty(ws_bytes + 1024, dtype=torch.uint8, device="cuda")
+    off = (-raw.data_ptr()) % 1024
+    ws_p = ctypes.c_void_p(raw.data_ptr() + off)
+    call("sglm_gram_tc_scaled_partial_f64", ptr(Xd), row_stride(Xd), ptr(Yd), row_stride(Yd), n_y, T, C, ptr(rs),
+         ptr(colE), ptr(colS), colS_p, 1, sizes_p, ptr(rows), 1, member.ctypes.data_as(ctypes.c_void_p), ws_p, ws_bytes,
+         stream_ptr())
+    all_reduce(raw[off + off_b.value: off + off_b.value + size_b.value].view(torch.int64), "sum")
+    G = _zeros((1, n_aug, ldg))
+    call("sglm_gram_tc_cells_combine_f64", C, n_y, ptr(colE), ptr(colS), colS_p, 1, sizes_p, 1, ptr(G), ldg, ws_p, ws_bytes,
+         stream_ptr())
+    return G
+
+
+def reduce_parts(parts, n_parts):
+    """parts: n_parts equal contiguous blocks -> their element-wise sum, added in block order (sglm_reduce_parts_f64):
+    the fixed-order sum of per-process partials gathered in process order."""
+    n = parts.numel() // n_parts
+    out = _empty((n,))
+    call("sglm_reduce_parts_f64", ptr(parts), n, int(n_parts), ptr(out), stream_ptr())
+    return out
+
+
 def poisson_irls(Xd, yd, alpha, fit_intercept=True, rw=None, max_iter=100, tol=1e-4, coef_init=None,
                  intercept_init=None):
     """argmin mean(mu - y*eta) + alpha/2 |w|^2 (rows weighted by multiplicity rw).
@@ -1254,11 +1316,12 @@ def _loss_name(power):
     return "HalfPoissonLoss" if power == 1 else "HalfTweedieLoss"
 
 
-def _pb_hessian(Xd, y_col, rw_vec, w_ref, b_ref, fit_intercept, n_tot, use_tc, power=1.0):
+def _pb_hessian(Xd, y_col, rw_vec, w_ref, b_ref, fit_intercept, n_tot, use_tc, power=1.0, comm=None):
     """H~ = X' diag(rw v_ref) X (centred on the weighted column means when an intercept is fitted) with the Fisher
     weights v_ref = mu_ref^(2-p) of one reference model: the fused row pass gives the weights, the tcgen05 digit-plane
     Gram (large problems) or the fp64 DMMA Gram the matrix.  Returns (Problem-like hess with Qc / xbar, h11 = sum of
-    the weights as a device scalar)."""
+    the weights as a device scalar).  With `comm` (rows sharded over processes, see tweedie_grid_batched) the Gram
+    is the staged one summed over the processes (tcgen05) or the combined fp64 partials, h11 the combined sum."""
     torch = nat.require_cuda()
     T, C = Xd.shape
     sums = _empty((8,))
@@ -1267,6 +1330,12 @@ def _pb_hessian(Xd, y_col, rw_vec, w_ref, b_ref, fit_intercept, n_tot, use_tc, p
     z = _empty((T, 1))
     call("sglm_glm_irls_prepare_f64", ptr(Xd), row_stride(Xd), ptr(y_col), ptr(rw_vec), T, C, ptr(w_ref), ptr(b_ref),
          float(power), ptr(weight), ptr(z), ptr(sums), ptr(ws), stream_ptr())
+    if comm is not None:
+        if use_tc:
+            G = suffstats_tc_scaled_sharded(Xd, z, weight[0].sqrt(), POISSON_TC_PLANES, comm.all_reduce)
+        else:
+            G = comm.combine(suffstats(Xd, z, weight, [n_tot]))
+        return center(G[0], None, C, 1, 0, fit_intercept), comm.combine(sums[1:2])
     if use_tc:
         G = suffstats_tc_scaled(Xd, z, weight[0].sqrt(), POISSON_TC_PLANES)
     else:
@@ -1282,10 +1351,16 @@ def poisson_grid_batched(Xd, Yd, models, RW=None):
     return tweedie_grid_batched(Xd, Yd, models, RW, 1.0)
 
 
-def tweedie_grid_batched(Xd, Yd, models, RW=None, power=1.0):
+def tweedie_grid_batched(Xd, Yd, models, RW=None, power=1.0, comm=None):
     """poisson_grid_batched for the Tweedie family of `power` (1, or > 1; log link): argmin mean(l(y, eta)) +
     alpha/2 |w|^2 with sklearn's HalfTweedieLoss l (p = 2: Gamma, whose Fisher Hessian X' diag(rw) X does not depend
-    on the iterate and is built once per fold)."""
+    on the iterate and is built once per fold).
+
+    comm: the rows are sharded over processes — Xd, Yd and RW hold this process's rows, every process calls with the
+    same models — and `comm` combines the cross-row reductions: all_reduce(t, op) in place for the integer
+    collectives of the tcgen05 Gram (op "max" / "min" / "sum"; also "min" on fp64), combine(t) = the fp64 partials
+    of all processes added in process order (every process gets the same bits).  Every process then holds every
+    model's coefficients; all host decisions are taken on combined values, so the processes stay in lock step."""
     torch = nat.require_cuda()
     global last_poisson_batch
     power = float(power)
@@ -1295,13 +1370,13 @@ def tweedie_grid_batched(Xd, Yd, models, RW=None, power=1.0):
     out_W, out_b, out_it, out_st = [], [], [], []
     diag = []
     for c0 in range(0, len(models), PB_MAX_BATCH):
-        Wb, bb, it, st, dg = _poisson_batch(Xd, Yd, models[c0:c0 + PB_MAX_BATCH], RW, power)
+        Wb, bb, it, st, dg = _poisson_batch(Xd, Yd, models[c0:c0 + PB_MAX_BATCH], RW, power, comm)
         out_W.append(Wb); out_b.append(bb); out_it.append(it); out_st.append(st); diag.append(dg)
     last_poisson_batch = diag
     return torch.cat(out_W), torch.cat(out_b), np.concatenate(out_it), np.concatenate(out_st)
 
 
-def _poisson_batch(Xd, Yd, models, RW, power):
+def _poisson_batch(Xd, Yd, models, RW, power, comm=None):
     torch = nat.require_cuda()
     T, C = Xd.shape
     B = len(models)
@@ -1314,7 +1389,17 @@ def _poisson_batch(Xd, Yd, models, RW, power):
     combos = sorted({(m.rw, m.ycol) for m in models})
     stats = torch.stack([torch.stack([(RW[rw].sum() if rw >= 0 else torch.tensor(float(T), device="cuda", dtype=torch.float64)),
                                       ((RW[rw] * Yd[:, yc]).sum() if rw >= 0 else Yd[:, yc].sum()),
-                                      Yd[:, yc].min()]) for rw, yc in combos]).cpu().numpy()
+                                      Yd[:, yc].min() if T else torch.tensor(np.inf, device="cuda", dtype=torch.float64)])
+                         for rw, yc in combos])
+    T_all = T
+    if comm is not None:
+        # counts and sums of y over all processes (+ the total row count, which picks the Hessian path), min y
+        sums_ = comm.combine(torch.cat([stats[:, :2].reshape(-1), torch.tensor([float(T)], device="cuda", dtype=torch.float64)]))
+        T_all = int(sums_[-1].item())
+        ymin = stats[:, 2].contiguous()
+        comm.all_reduce(ymin, "min")
+        stats = torch.cat([sums_[:-1].reshape(-1, 2), ymin[:, None]], dim=1)
+    stats = stats.cpu().numpy()
     info = {k: v for k, v in zip(combos, stats)}
     if any(v[2] < 0 for v in info.values()) or any(not (v[1] > 0) for v in info.values()) or \
             (power >= 2 and any(not (v[2] > 0) for v in info.values())):
@@ -1349,8 +1434,9 @@ def _poisson_batch(Xd, Yd, models, RW, power):
     hess_id = _dev([gkeys.index((m.rw, m.fit_intercept)) for m in models], i32)
     ycol = _dev([m.ycol for m in models], i32)
     rw_a = _dev([m.rw for m in models], i32)
-    sums = _zeros((B, 4))
-    Gw = _zeros((C, ldb))
+    red = _zeros((C * ldb + B * 4,))        # the cross-row reductions of an iteration, combined in one call under comm
+    Gw = red[:C * ldb].view(C, ldb)
+    sums = red[C * ldb:].view(B, 4)
     Wt = _zeros((C, ldb))
     Eta = _empty((max(T, 1), ldb))
     xt_bytes = nat.lib().sglm_pb_gemm_tn_workspace_bytes(T, C, ldb)
@@ -1359,7 +1445,7 @@ def _poisson_batch(Xd, Yd, models, RW, power):
     ep_ws = torch.empty(ep_bytes // 8 + 1, dtype=torch.float64, device="cuda")
     ldq = _round_up(C, 8)
     # ---- Hessians (one per fold / intercept setting) and the factors of (H~ + alpha n I) of every model
-    use_tc = _poisson_tc(T, C)
+    use_tc = _poisson_tc(T_all, C)
     n_h = len(gkeys)
     HQ = torch.zeros(n_h, dtype=torch.int64, device="cuda")
     Hxbar = torch.zeros(n_h, dtype=torch.int64, device="cuda")
@@ -1377,7 +1463,7 @@ def _poisson_batch(Xd, Yd, models, RW, power):
         idxs = groups[gkeys[g]]
         rw_vec = RW[rw] if rw >= 0 else None
         hess, h11 = _pb_hessian(Xd, ycontig[models[ref].ycol], rw_vec, W[ref], b[ref:ref + 1], fi, float(n_tot[ref]), use_tc,
-                                power)
+                                power, comm)
         an = _dev([models[i].alpha * n_tot[i] for i in idxs], f64)
         wb = nat.lib().sglm_ridge_workspace_bytes(C, hess.ldq, len(idxs))
         work = torch.empty(wb // 8, dtype=torch.float64, device="cuda")
@@ -1449,6 +1535,8 @@ def _poisson_batch(Xd, Yd, models, RW, power):
              ptr(status), power, 0, ptr(sums), ptr(ep_ws), ep_ws.numel() * 8, stream_ptr())
         call("sglm_pb_xt_r_f64", ptr(Xd), row_stride(Xd), T, C, ptr(Eta), ldb, ptr(Gw), ptr(xt_ws), xt_ws.numel() * 8,
              stream_ptr())
+        if comm is not None:
+            red.copy_(comm.combine(red))
         call("sglm_pb_step_f64", state_p, ptr(L_of), stream_ptr())
         it += 1
         host = torch.stack([status.to(torch.float64), step_out, ratio_out]).cpu().numpy()     # the one read-back per iteration
@@ -1486,9 +1574,10 @@ def poisson_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW):
     return tweedie_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW, 1.0)
 
 
-def tweedie_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW, power):
+def tweedie_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW, power, comm=None):
     """poisson_scores_batched for the Tweedie family of `power`: slots 4..6 hold the family's deviance terms
-    (sglm_score_glm_f64 semantics), the input of tweedie_d2_from_sums."""
+    (sglm_score_glm_f64 semantics), the input of tweedie_d2_from_sums.  comm: rows sharded over processes, the sums
+    combined (tweedie_grid_batched)."""
     torch = nat.require_cuda()
     T, C = Xd.shape
     B = W.shape[0]
@@ -1510,5 +1599,7 @@ def tweedie_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW, power):
              ptr(RW) if RW is not None else None, RW.stride(0) if RW is not None else 0,
              ptr(ids[1]), ptr(ids[2]), ptr(b_part), None, float(power), 1, ptr(sums), ptr(ep_ws), ep_ws.numel() * 8,
              stream_ptr())
+        if comm is not None:
+            sums = comm.combine(sums)
         out[c0:c0 + n] = sums.cpu().numpy().reshape(n, 2, 8)
     return out

@@ -60,6 +60,10 @@ _PROTOTYPES = {
     "sglm_gram_tc_cells_sgout": (c_i32, [c_i32, c_vp, c_i32, c_vp, c_i32, c_vp, c_vp]),
     "sglm_gram_tc_cells_partial_f64": (c_i32, [c_vp, c_i64, c_vp, c_i64, c_i32, c_i64, c_i32, c_vp, c_vp, c_vp, c_i32,
                                                c_vp, c_vp, c_i32, c_vp, c_vp, c_sz, c_vp]),
+    "sglm_gram_tc_colstats_scaled_f64": (c_i32, [c_vp, c_i64, c_vp, c_i64, c_i32, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp]),
+    "sglm_gram_tc_scaled_partial_f64": (c_i32, [c_vp, c_i64, c_vp, c_i64, c_i32, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp,
+                                                c_i32, c_vp, c_vp, c_i32, c_vp, c_vp, c_sz, c_vp]),
+    "sglm_reduce_parts_f64": (c_i32, [c_vp, c_i64, c_i32, c_vp, c_vp]),
     "sglm_gram_tc_cells_combine_f64": (c_i32, [c_i32, c_i32, c_vp, c_vp, c_vp, c_i32, c_vp, c_i32, c_vp, c_i64, c_vp,
                                                c_sz, c_vp]),
     "sglm_index_counts_f64": (c_i32, [c_vp, c_i64, c_vp, c_i64, c_vp]),
@@ -165,7 +169,7 @@ def ptr(t):
 
 # kernels launched per ABI call (for the launch count bench.py reports)
 _KERNELS_PER_CALL = {"sglm_suffstats_f64": 3, "sglm_gram_tc_analyze_f64": 2, "sglm_gram_tc_f64": 4, "sglm_gram_tc_cells_f64": 5,
-                     "sglm_gram_tc_lag_cells_f64": 7, "sglm_gram_tc_cells_partial_f64": 4, "sglm_gram_tc_scaled_f64": 4,
+                     "sglm_gram_tc_lag_cells_f64": 7, "sglm_gram_tc_cells_partial_f64": 4, "sglm_gram_tc_scaled_partial_f64": 4, "sglm_gram_tc_scaled_f64": 4,
                      "sglm_gram_tc_analyze_scaled_f64": 2, "sglm_quadform_gemm_f64": 3, "sglm_xt_vec_f64": 2, "sglm_score_f64": 2,
                      "sglm_poisson_irls_prepare_f64": 2, "sglm_timeshift_f64": 2, "sglm_pb_xt_r_f64": 2, "sglm_pb_epilogue_f64": 2,
                      "sglm_glm_epilogue_f64": 2, "sglm_score_glm_f64": 2, "sglm_glm_irls_prepare_f64": 2,

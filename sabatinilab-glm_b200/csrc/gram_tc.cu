@@ -910,10 +910,8 @@ extern "C" int sglm_gram_tc_analyze_f64(const double *X, int64_t ldx, const doub
 // them (max / min: an all-reduce of 2 * n_aug integers), and every rank derives the same exponents and digit-plane
 // counts — so the integer digit planes, and the int64 plane Grams that are then summed over the ranks, are those of
 // the one-GPU computation bit for bit.
-extern "C" int sglm_gram_tc_colstats_f64(const double *X, int64_t ldx, const double *Y, int64_t ldy, int32_t n_y,
-                                         int64_t T, int32_t C, uint64_t *colmax_bits, int32_t *col_lsb, void *stream) {
-    SGLM_CHECK_ARG(T >= 0 && C >= 0 && n_y >= 0 && ldx >= C && ldy >= n_y, SGLM_E_SHAPE, "gram_tc_colstats: bad shape");
-    SGLM_CHECK_ARG(colmax_bits && col_lsb, SGLM_E_INVALID_ARG, "gram_tc_colstats: null pointer");
+static int gram_tc_colstats(const double *X, int64_t ldx, const double *Y, int64_t ldy, int32_t n_y, int64_t T,
+                            int32_t C, const double *rs, uint64_t *colmax_bits, int32_t *col_lsb, void *stream) {
     cudaStream_t st = (cudaStream_t)stream;
     const int n_aug = C + n_y + 1;
     SGLM_CUDA_OK(cudaMemsetAsync(colmax_bits, 0, (size_t)n_aug * sizeof(uint64_t), st));
@@ -921,10 +919,27 @@ extern "C" int sglm_gram_tc_colstats_f64(const double *X, int64_t ldx, const dou
     if (T > 0) {
         const int gy = (int)std::max<long long>(1, std::min<long long>(T / 256, 64LL * sm_count() / std::max(1, ceil_div(n_aug, 256))));
         dim3 grid(ceil_div(n_aug, 256), gy);
-        tc_colmax_kernel<<<grid, 256, 0, st>>>(X, ldx, Y, ldy, C, n_y, T, nullptr, (unsigned long long *)colmax_bits, col_lsb);
+        tc_colmax_kernel<<<grid, 256, 0, st>>>(X, ldx, Y, ldy, C, n_y, T, rs, (unsigned long long *)colmax_bits, col_lsb);
         SGLM_LAUNCH_OK("tc_colmax_kernel");
     }
     return SGLM_OK;
+}
+
+extern "C" int sglm_gram_tc_colstats_f64(const double *X, int64_t ldx, const double *Y, int64_t ldy, int32_t n_y,
+                                         int64_t T, int32_t C, uint64_t *colmax_bits, int32_t *col_lsb, void *stream) {
+    SGLM_CHECK_ARG(T >= 0 && C >= 0 && n_y >= 0 && ldx >= C && ldy >= n_y, SGLM_E_SHAPE, "gram_tc_colstats: bad shape");
+    SGLM_CHECK_ARG(colmax_bits && col_lsb, SGLM_E_INVALID_ARG, "gram_tc_colstats: null pointer");
+    return gram_tc_colstats(X, ldx, Y, ldy, n_y, T, C, nullptr, colmax_bits, col_lsb, stream);
+}
+
+// The column pass of the weighted Gram (rows scaled by row_scale, as in sglm_gram_tc_analyze_scaled_f64) over THIS
+// rank's rows; sglm_gram_tc_exponents with the Gram's max_planes finishes the analysis after the ranks' max / min.
+extern "C" int sglm_gram_tc_colstats_scaled_f64(const double *X, int64_t ldx, const double *Y, int64_t ldy, int32_t n_y,
+                                                int64_t T, int32_t C, const double *row_scale, uint64_t *colmax_bits,
+                                                int32_t *col_lsb, void *stream) {
+    SGLM_CHECK_ARG(T >= 0 && C >= 0 && n_y >= 0 && ldx >= C && ldy >= n_y, SGLM_E_SHAPE, "gram_tc_colstats_scaled: bad shape");
+    SGLM_CHECK_ARG(colmax_bits && col_lsb && (row_scale || T == 0), SGLM_E_INVALID_ARG, "gram_tc_colstats_scaled: null pointer");
+    return gram_tc_colstats(X, ldx, Y, ldy, n_y, T, C, row_scale, colmax_bits, col_lsb, stream);
 }
 
 // colS holds the (combined) lowest set bits on entry and the digit-plane counts on exit.
@@ -1062,6 +1077,24 @@ extern "C" int sglm_gram_tc_cells_partial_f64(const double *X, int64_t ldx, cons
     double dummy;
     return gram_tc_run(X, ldx, Y, ldy, n_y, T, C, colE, colS, colS_host, n_cells, cell_rows_host, rows, n_out,
                        member_host, &dummy, C + n_y + 1, workspace, workspace_bytes, 0, stream, nullptr, 1);
+}
+
+// Weighted form of sglm_gram_tc_cells_partial_f64 (rows of Z scaled by row_scale; colE / colS from
+// sglm_gram_tc_colstats_scaled_f64 + sglm_gram_tc_exponents with the Gram's max_planes): a rank's share of
+// Z' diag(row_scale^2) Z as int64 plane Grams.  The digits of a row depend only on that row and the combined analysis,
+// so the partials summed over ANY partition of the rows and then combined are the bits of sglm_gram_tc_scaled_f64.
+extern "C" int sglm_gram_tc_scaled_partial_f64(const double *X, int64_t ldx, const double *Y, int64_t ldy, int32_t n_y,
+                                               int64_t T, int32_t C, const double *row_scale, const int32_t *colE,
+                                               const int32_t *colS, const int32_t *colS_host, int32_t n_cells,
+                                               const int64_t *cell_rows_host, const int64_t *rows, int32_t n_out,
+                                               const int32_t *member_host, void *workspace, size_t workspace_bytes,
+                                               void *stream) {
+    SGLM_CHECK_ARG(n_out >= 1 && member_host, SGLM_E_INVALID_ARG, "gram_tc_scaled_partial: membership table missing");
+    SGLM_CHECK_ARG(n_cells <= TC_SUM_CELLS, SGLM_E_UNSUPPORTED, "gram_tc_scaled_partial: at most %d cells", TC_SUM_CELLS);
+    SGLM_CHECK_ARG(row_scale || T == 0, SGLM_E_INVALID_ARG, "gram_tc_scaled_partial: null row_scale");
+    double dummy;
+    return gram_tc_run(X, ldx, Y, ldy, n_y, T, C, colE, colS, colS_host, n_cells, cell_rows_host, rows, n_out,
+                       member_host, &dummy, C + n_y + 1, workspace, workspace_bytes, 0, stream, row_scale, 1);
 }
 
 extern "C" int sglm_gram_tc_cells_combine_f64(int32_t C, int32_t n_y, const int32_t *colE, const int32_t *colS,

@@ -495,6 +495,18 @@ extern "C" int sglm_pb_xt_r_f64(const double *X, int64_t ldx, int64_t T, int32_t
     return SGLM_OK;
 }
 
+// out[e] = sum over k = 0, 1, ... of parts[k][e], added in that order: the per-rank partial sums of a row-sharded
+// batch, gathered in rank order, give the same bits on every rank.
+extern "C" int sglm_reduce_parts_f64(const double *parts, int64_t n_elem, int32_t n_parts, double *out, void *stream) {
+    SGLM_CHECK_ARG(n_elem >= 0 && n_parts >= 1, SGLM_E_SHAPE, "reduce_parts: bad shape");
+    if (n_elem == 0) return SGLM_OK;
+    SGLM_CHECK_ARG(parts && out, SGLM_E_INVALID_ARG, "reduce_parts: null pointer");
+    pb_reduce_splits_kernel<<<(unsigned)std::min<long long>(ceil_div<long long>(n_elem, 256), sm_count() * 8LL), 256, 0,
+                              (cudaStream_t)stream>>>(parts, n_elem, n_parts, out);
+    SGLM_LAUNCH_OK("pb_reduce_splits_kernel");
+    return SGLM_OK;
+}
+
 static int pb_epi_grid(long long T) { return (int)std::max<long long>(1, std::min<long long>(sm_count() * 8LL, ceil_div<long long>(T, 64))); }
 
 extern "C" size_t sglm_pb_epilogue_workspace_bytes(int64_t T, int32_t n_models) {

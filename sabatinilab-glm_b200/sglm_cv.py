@@ -515,6 +515,14 @@ def _poisson_grid(Xd, yd, cv_idx, glms, rolls, score_method, power=1.0):
         if r % max(T, 1) == 0:
             ycol_of_roll[r] = 0
     Yd = torch.stack([yd if k == 0 else eng.roll_vector(yd, int(r)) for k, r in enumerate(roll_vals)], dim=1).contiguous()
+    return _tweedie_cv(Xd, Yd, ycol_of_roll, RW, F, glms, rolls, score_method, power)
+
+
+def _tweedie_cv(Xd, Yd, ycol_of_roll, RW, F, glms, rolls, score_method, power, comm=None):
+    """The batched fits and scores of _poisson_grid from its inputs: the response columns Yd (one per distinct roll,
+    column 0 un-rolled), the row weights RW (rows 0..F-1 train, F..2F-1 test).  comm: the rows are sharded over
+    processes (sglm_dist.cv_grid_strong; see _engine.tweedie_grid_batched) — every process returns the same results."""
+    C = Xd.shape[1]
     models, ycol, rw_a, rw_b = [], [], [], []
     for glm, r in zip(glms, rolls):
         est = glm.model
@@ -525,8 +533,8 @@ def _poisson_grid(Xd, yd, cv_idx, glms, rolls, score_method, power=1.0):
             ycol.append(ycol_of_roll[r]); rw_a.append(f); rw_b.append(F + f)
         models.append(eng.PoissonModel(est.alpha, est.fit_intercept, rw=-1, ycol=0, max_iter=est.max_iter, tol=est.tol))
         ycol.append(0); rw_a.append(-1); rw_b.append(-2)          # the refit uses the UN-rolled y (backend/sglm_cv.py:181)
-    Wd, bd, n_it, status = eng.tweedie_grid_batched(Xd, Yd, models, RW, power)
-    sums = eng.tweedie_scores_batched(Xd, Yd, Wd, bd, ycol, rw_a, rw_b, RW, power)
+    Wd, bd, n_it, status = eng.tweedie_grid_batched(Xd, Yd, models, RW, power, comm)
+    sums = eng.tweedie_scores_batched(Xd, Yd, Wd, bd, ycol, rw_a, rw_b, RW, power, comm)
     W_h, b_h = Wd.cpu().numpy(), bd.cpu().numpy()
     results = []
     for k, glm in enumerate(glms):

@@ -201,6 +201,35 @@ def unpack_results(gathered, owner_lists, C):
     return full
 
 
+class RankComm:
+    """The cross-row reductions of a row-sharded computation over the ranks of `group` (NCCL, device tensors):
+    all_reduce(t, op) in place (op "max" / "min" / "sum"), and combine(t) = the fp64 tensors of all ranks gathered and
+    added in rank order on the device (_engine.reduce_parts) — every rank gets the same bits, which an fp64 all-reduce
+    does not promise."""
+
+    def __init__(self, group=None):
+        dist = _dist()
+        self.group = group
+        self.world = dist.get_world_size(group)
+
+    def all_reduce(self, t, op):
+        dist = _dist()
+        dist.all_reduce(t, op={"max": dist.ReduceOp.MAX, "min": dist.ReduceOp.MIN, "sum": dist.ReduceOp.SUM}[op],
+                        group=self.group)
+
+    def combine(self, t):
+        import torch
+        import _engine as eng
+        flat = t.reshape(-1).contiguous()
+        parts = torch.empty(self.world * flat.numel(), dtype=flat.dtype, device=flat.device)
+        _dist().all_gather_into_tensor(parts, flat, group=self.group)
+        return eng.reduce_parts(parts, self.world).reshape(t.shape)
+
+
+LOG_LINK_KINDS = ("poisson", "tweedie")
+GAUSSIAN_KINDS = ("ols", "ridge", "lasso", "enet")
+
+
 def cv_grid_strong(X0, shift_amt_list, y, cv_idx, model_name, glm_kwarg_lst, verbose=0, score_method='mse',
                    rows=None, shift_inx=[], fill_value=np.nan, group=None, src=0):
     """`sglm_pp.timeshift_multiple(X0, shift_inx, shift_amt_list)[rows] -> sglm_cv.cv_glm_mult_params(design, y,
@@ -214,8 +243,15 @@ def cv_grid_strong(X0, shift_amt_list, y, cv_idx, model_name, glm_kwarg_lst, ver
       fits        models dealt to the ranks by cost; each rank runs its share of the batched plan
       results     one packed all_gather of [coef | intercept | RSS | info]; selection on every rank
 
+    Poisson, Gamma and Tweedie sets (log link) run the batched IRLS of sglm_cv, one batch per distinct power, on the
+    rows [g0, g1) of this rank's slice of the design: every cross-row sum of an iteration (objective and gradient
+    sums, X'R, the weighted Hessian Gram, the scores) is combined over the ranks (RankComm), so every rank runs every
+    log-link model in lock step and holds all their coefficients.  Unlike the Gaussian statistics, the fp64 gradient
+    sums are re-associated over the ranks: the log-link results agree with the one-GPU grid to rounding, not to the bit.
+
     rows = (lo, hi): base rows kept after `dropna` (default: the rows without NaN padding).  Folds must be the
-    usual complement pairs with duplicate-free test rows (cv_idx_by_*); Gaussian family."""
+    usual complement pairs with duplicate-free test rows (cv_idx_by_*); Gaussian, Poisson, Gamma and Tweedie
+    families, mixed in one call."""
     import torch
     import _engine as eng
     import sglm_
@@ -279,12 +315,12 @@ def cv_grid_strong(X0, shift_amt_list, y, cv_idx, model_name, glm_kwarg_lst, ver
     g0, g1 = n * rank // world, n * (rank + 1) // world
     src_cols, sh_cols, _ = sglm_pp.build_column_map(P, shift_inx, shifts)
     # ... as a recipe: the statistics come from the base signals (eng.LagRecipe), the slice of the design is only built
-    # when a column reads outside the base signals
+    # when a column reads outside the base signals or a log-link family needs it for its GEMMs
     Xd = eng.LagRecipe(X0d, src_cols, sh_cols, lo + g0, lo + g1, fill_value)
     C = Xd.shape[1]
     mark("gather")
 
-    # ---- parameter sets -> estimators (identical on every rank)
+    # ---- parameter sets -> estimators (identical on every rank: every raise below happens on every rank)
     entries = []
     for kw in glm_kwarg_lst:
         name = kw.pop('model_name', 'Gaussian')                    # backend/sglm_cv.py:288
@@ -293,53 +329,90 @@ def cv_grid_strong(X0, shift_amt_list, y, cv_idx, model_name, glm_kwarg_lst, ver
     for name, kw in entries:
         rolls.append(int(kw.pop('roll', 0)))                       # backend/sglm_cv.py:95
         glms.append(sglm_.GLM(name, **kw))
-        if glms[-1].model.kind not in ("ols", "ridge", "lasso", "enet"):
-            raise NotImplementedError("cv_grid_strong: Gaussian family")
-    roll_vals = [0] + sorted({r for r in rolls if r % max(n, 1) != 0})
-    ycols = [yd if k == 0 else eng.roll_vector(yd, int(r)) for k, r in enumerate(roll_vals)]
-    Yd = torch.stack([c[g0:g1] for c in ycols], dim=1).contiguous()
+        if glms[-1].model.kind not in GAUSSIAN_KINDS + LOG_LINK_KINDS:
+            raise NotImplementedError("cv_grid_strong: Gaussian, Poisson, Gamma and Tweedie (log link) families")
+    gauss = [i for i, g in enumerate(glms) if g.model.kind in GAUSSIAN_KINDS]
+    by_power = {}                                                  # one batch per distinct power, as sglm_cv._cv_batch
+    for i, g in enumerate(glms):
+        if g.model.kind in LOG_LINK_KINDS:
+            by_power.setdefault(1.0 if g.model.kind == "poisson" else g.model.power, []).append(i)
     # ---- this rank's part of every test list (sorted global lists -> local row numbers)
     bounds = torch.tensor([g0, g1], dtype=torch.int64, device=dev)
     local_tests = []
     for t in tests:
         cut = torch.searchsorted(t, bounds).cpu().numpy()
         local_tests.append(t[int(cut[0]):int(cut[1])] - g0)
+    comm = RankComm(group)
 
-    def all_reduce(t, op):
-        dist.all_reduce(t, op={"max": dist.ReduceOp.MAX, "min": dist.ReduceOp.MIN, "sum": dist.ReduceOp.SUM}[op], group=group)
+    def y_columns(rs):
+        """The local rows of y and of its rolled copies (rolled over ALL rows), column 0 un-rolled."""
+        roll_vals = [0] + sorted({r for r in rs if r % max(n, 1) != 0})
+        ycol_of_roll = {r: k for k, r in enumerate(roll_vals)}
+        for r in rs:
+            if r % max(n, 1) == 0:
+                ycol_of_roll[r] = 0
+        cols = [yd if k == 0 else eng.roll_vector(yd, int(r)) for k, r in enumerate(roll_vals)]
+        return torch.stack([c[g0:g1] for c in cols], dim=1).contiguous(), ycol_of_roll
 
-    G = eng.suffstats_tc_sharded(Xd, Yd, [None] + local_tests, all_reduce)
-    mark("statistics")
+    out = [None] * len(glms)
+    mine = []
+    if gauss:
+        g_glms, g_rolls = [glms[i] for i in gauss], [rolls[i] for i in gauss]
+        Yd, _ = y_columns(g_rolls)
+        G = eng.suffstats_tc_sharded(Xd, Yd, [None] + local_tests, comm.all_reduce)
+        mark("statistics")
+
+        ses = sglm_cv.GaussianSession.from_statistics(G, n, C, yd, n_te, g_glms, g_rolls, score_method)
+        models = ses.model_specs()
+        M = len(models)
+        owner, _ = deal_models([model_cost(s) for s in models], world)
+        owner_lists = [np.flatnonzero(owner == r) for r in range(world)]
+        mine = owner_lists[rank]
+        mark("problems")
+        W, info, status = eng.solve_models([models[i] for i in mine], C)
+        mark("fits")
+        b_d, rss_full, rss_test, rss_train = ses.score(W, mine)
+        n_pad = max(len(o) for o in owner_lists) if M else 0
+        mine_pack = pack_results(W[:, :C], b_d, rss_full, rss_test, rss_train, info, status, n_pad)
+        gathered = torch.empty((world, n_pad, C + 11), dtype=torch.float64, device=dev)
+        dist.all_gather_into_tensor(gathered.reshape(world * n_pad, C + 11), mine_pack, group=group)
+        mark("scores+all_gather")
+        full = unpack_results(gathered, owner_lists, C)
+
+        n_sets = len(g_glms)
+        W3 = full[:, :C].reshape(n_sets, F + 1, C)
+        coef_folds = W3[:, :F, :].permute(0, 2, 1).contiguous().cpu().numpy()
+        coef_full = W3[:, F, :].contiguous().cpu().numpy()
+        tail = full[:, C:].cpu().numpy()
+        res = ses.assemble(coef_folds, coef_full, tail[:, 0].copy(), tail[:, 2].copy(), tail[:, 3].copy(),
+                           tail[:, 4:10].copy(), tail[:, 10].astype(np.int64))
+        for i, r in zip(gauss, res):
+            out[i] = r
+        mark("download+assemble")
+    if by_power:
+        # the log-link families: this rank's rows of the design for the two GEMMs of every iteration, its rows of the
+        # train / test weights (complement folds: train = 1 - test), the finiteness check combined over the ranks
+        Xl = Xd.tensor()
+        finite = torch.isfinite(Xl).all().to(torch.int32).reshape(1)
+        comm.all_reduce(finite, "min")
+        if not bool(finite.item()):
+            raise ValueError("Input X contains NaN or infinity.")
+        te_w = [eng.index_counts(t, g1 - g0) for t in local_tests]
+        RW = torch.stack([1.0 - w for w in te_w] + te_w).contiguous() if F else None
+        mark("loglink_design")
+        for power, idx in by_power.items():
+            l_rolls = [rolls[i] for i in idx]
+            Yl, ycol_of_roll = y_columns(l_rolls)
+            res = sglm_cv._tweedie_cv(Xl, Yl, ycol_of_roll, RW, F, [glms[i] for i in idx], l_rolls, score_method,
+                                      power, comm)
+            for i, r in zip(idx, res):
+                out[i] = r
+            mark(f"loglink_fits_power_{power:g}")
+        del Xl, RW
     del Xd
-
-    ses = sglm_cv.GaussianSession.from_statistics(G, n, C, yd, n_te, glms, rolls, score_method)
-    models = ses.model_specs()
-    M = len(models)
-    owner, _ = deal_models([model_cost(s) for s in models], world)
-    owner_lists = [np.flatnonzero(owner == r) for r in range(world)]
-    mine = owner_lists[rank]
-    mark("problems")
-    W, info, status = eng.solve_models([models[i] for i in mine], C)
-    mark("fits")
-    b_d, rss_full, rss_test, rss_train = ses.score(W, mine)
-    n_pad = max(len(o) for o in owner_lists) if M else 0
-    mine_pack = pack_results(W[:, :C], b_d, rss_full, rss_test, rss_train, info, status, n_pad)
-    gathered = torch.empty((world, n_pad, C + 11), dtype=torch.float64, device=dev)
-    dist.all_gather_into_tensor(gathered.reshape(world * n_pad, C + 11), mine_pack, group=group)
-    mark("scores+all_gather")
-    full = unpack_results(gathered, owner_lists, C)
-
-    n_sets = len(glms)
-    W3 = full[:, :C].reshape(n_sets, F + 1, C)
-    coef_folds = W3[:, :F, :].permute(0, 2, 1).contiguous().cpu().numpy()
-    coef_full = W3[:, F, :].contiguous().cpu().numpy()
-    tail = full[:, C:].cpu().numpy()
-    res = ses.assemble(coef_folds, coef_full, tail[:, 0].copy(), tail[:, 2].copy(), tail[:, 3].copy(),
-                       tail[:, 4:10].copy(), tail[:, 10].astype(np.int64))
-    for (name, kw), r in zip(entries, res):
+    for (name, kw), r in zip(entries, out):
         r['glm_kwargs'] = kw
-    mark("download+assemble")
     torch.cuda.synchronize()
     last_timeline = {name: float(ev[k - 1][1].elapsed_time(e)) for k, (name, e) in enumerate(ev) if k > 0}
     last_timeline["models_on_this_rank"] = int(len(mine))
-    return sglm_cv._select_best([sglm_cv._order_result(r) for r in res], score_method)
+    return sglm_cv._select_best([sglm_cv._order_result(r) for r in out], score_method)
