@@ -481,7 +481,12 @@ int sglm_pb_epilogue_f64(double *Eta, int64_t ldb, int32_t n_models, int64_t T, 
                          void *workspace, size_t workspace_bytes, void *stream);
 /* sglm_pb_epilogue_f64 for the Tweedie family of `power` (1, or > 1 — else SGLM_E_UNSUPPORTED before any CUDA call;
  * log link): mode 0 writes R = rw dloss/deta = rw mu^(1-p) (mu - y) and sums [B][4] = {sum rw loss, sum rw mu^(2-p),
- * sum rw, sum R}; mode 1 the sglm_score_glm_f64 sums.  power = 1 is sglm_pb_epilogue_f64. */
+ * sum rw, sum R}; mode 1 the sglm_score_glm_f64 sums.  power = 1 is sglm_pb_epilogue_f64.
+ * RW is not checked: a model with rw_a (or, in mode 1, rw_b) >= 0 reads RW row rw_a, so RW = NULL is only valid
+ * when T = 0 or every id is negative.  T = 0 (an empty row slice) accepts Eta = Y = NULL and writes zero sums; the
+ * same holds for X / R of sglm_pb_xt_r_f64 (Gw = 0), X / r of sglm_xt_vec_f64 (out = 0) and X / y / resid / weight /
+ * z of sglm_score_glm_f64 and sglm_glm_irls_prepare_f64.  sglm_pb_xt_r_f64 needs R and its workspace 16-byte
+ * aligned. */
 int sglm_glm_epilogue_f64(double *Eta, int64_t ldb, int32_t n_models, int64_t T, const double *Y, int64_t ldy,
                           const int32_t *ycol, const double *RW, int64_t ldrw, const int32_t *rw_a,
                           const int32_t *rw_b, const double *b, const int32_t *status, double power, int32_t mode,

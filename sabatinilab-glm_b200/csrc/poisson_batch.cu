@@ -475,11 +475,13 @@ extern "C" int sglm_quadform_gemm_f64(const double *A, int64_t lda, int32_t n, c
     return SGLM_OK;
 }
 
-// Gw [C][ldb] = X' R   (R [T][ldb]); deterministic: fixed T chunks of 8192 rows, partials added in order
+// Gw [C][ldb] = X' R   (R [T][ldb]); deterministic: fixed T chunks of 8192 rows, partials added in order.
+// T = 0 (an empty row slice): X and R may be null, Gw = 0.
 extern "C" int sglm_pb_xt_r_f64(const double *X, int64_t ldx, int64_t T, int32_t C, const double *R, int64_t ldb,
                                 double *Gw, void *workspace, size_t workspace_bytes, void *stream) {
     SGLM_CHECK_ARG(T >= 0 && C > 0 && ldx >= C && ldb >= 64 && ldb % 64 == 0, SGLM_E_SHAPE, "pb_xt_r: bad shape");
-    SGLM_CHECK_ARG(X && R && Gw && workspace, SGLM_E_INVALID_ARG, "pb_xt_r: null pointer");
+    SGLM_CHECK_ARG((T == 0 || (X && R)) && Gw && workspace, SGLM_E_INVALID_ARG, "pb_xt_r: null pointer");
+    SGLM_CHECK_ARG(((uintptr_t)R & 15) == 0 && ((uintptr_t)workspace & 15) == 0, SGLM_E_ALIGN, "pb_xt_r: 16-byte alignment");
     SGLM_CHECK_ARG(workspace_bytes >= sglm_pb_gemm_tn_workspace_bytes(T, C, ldb), SGLM_E_WORKSPACE, "pb_xt_r: workspace too small");
     const long long rows_per = 8192;
     const int n_split = (int)std::max<long long>(1, ceil_div<long long>(std::max<long long>(T, 1), rows_per));
@@ -534,8 +536,10 @@ static int pb_epilogue(const char *name, double *Eta, int64_t ldb, int32_t n_mod
                        const int32_t *rw_b, const double *b, const int32_t *status, double power, int32_t mode,
                        double *sums, void *workspace, size_t workspace_bytes, void *stream) {
     SGLM_CHECK_ARG(T >= 0 && n_models > 0 && ldb >= n_models && ldy >= 1, SGLM_E_SHAPE, "%s: bad shape", name);
-    SGLM_CHECK_ARG(Eta && Y && ycol && rw_a && b && sums && workspace && (mode == 0 || rw_b), SGLM_E_INVALID_ARG,
-                   "%s: null pointer", name);
+    // T = 0 (an empty row slice): no row is read or written, Eta, Y and RW may be null and the sums are 0.  RW is not
+    // checked: with T > 0 it must hold every row-weight vector an rw id >= 0 names.
+    SGLM_CHECK_ARG((T == 0 || (Eta && Y)) && ycol && rw_a && b && sums && workspace && (mode == 0 || rw_b),
+                   SGLM_E_INVALID_ARG, "%s: null pointer", name);
     SGLM_CHECK_ARG(glm_power_ok(power), SGLM_E_UNSUPPORTED, "%s: power %g (supported: 1 and > 1, log link)", name, power);
     SGLM_CHECK_ARG(workspace_bytes >= sglm_pb_epilogue_workspace_bytes(T, n_models), SGLM_E_WORKSPACE,
                    "%s: workspace too small", name);

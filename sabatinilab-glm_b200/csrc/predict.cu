@@ -253,11 +253,13 @@ extern "C" int sglm_score_f64(const double *X, int64_t ldx, const double *y, con
                                                   workspace, stream);
 }
 
+// The Tweedie family of `power` (sglm_b200.h).  T = 0 (an empty row slice): X, y and the row outputs may be null, the
+// sums are 0.
 extern "C" int sglm_score_glm_f64(const double *X, int64_t ldx, const double *y, const double *rw, int64_t T,
                                   int32_t C, const double *w, const double *b_dev, double power, double *resid,
                                   double *sums, void *workspace, void *stream) {
     SGLM_CHECK_ARG(T >= 0 && C > 0 && ldx >= C, SGLM_E_SHAPE, "score_glm: bad shape");
-    SGLM_CHECK_ARG(X && y && w && sums && workspace, SGLM_E_INVALID_ARG, "score_glm: null pointer");
+    SGLM_CHECK_ARG((T == 0 || (X && y)) && w && sums && workspace, SGLM_E_INVALID_ARG, "score_glm: null pointer");
     SGLM_CHECK_ARG(glm_power_ok(power), SGLM_E_UNSUPPORTED, "score_glm: power %g (supported: 1 and > 1, log link)", power);
     SGLM_CHECK_ARG((size_t)((C + 1) & ~1) * sizeof(double) <= 200 * 1024, SGLM_E_UNSUPPORTED, "score_glm: C=%d too large", C);
     return row_pass_sums_family<MODE_SCORE>(X, ldx, y, rw, T, C, w, b_dev, 1, power, resid, nullptr, sums, workspace,
@@ -279,7 +281,8 @@ extern "C" int sglm_glm_irls_prepare_f64(const double *X, int64_t ldx, const dou
                                          int64_t T, int32_t C, const double *w, const double *b_dev, double power,
                                          double *weight, double *z, double *sums, void *workspace, void *stream) {
     SGLM_CHECK_ARG(T >= 0 && C > 0 && ldx >= C, SGLM_E_SHAPE, "glm_irls_prepare: bad shape");
-    SGLM_CHECK_ARG(X && y && w && weight && z && sums && workspace, SGLM_E_INVALID_ARG, "glm_irls_prepare: null pointer");
+    SGLM_CHECK_ARG((T == 0 || (X && y && weight && z)) && w && sums && workspace, SGLM_E_INVALID_ARG,
+                   "glm_irls_prepare: null pointer");
     SGLM_CHECK_ARG(glm_power_ok(power), SGLM_E_UNSUPPORTED, "glm_irls_prepare: power %g (supported: 1 and > 1, log link)",
                    power);
     SGLM_CHECK_ARG((size_t)((C + 1) & ~1) * sizeof(double) <= 200 * 1024, SGLM_E_UNSUPPORTED,
@@ -289,11 +292,12 @@ extern "C" int sglm_glm_irls_prepare_f64(const double *X, int64_t ldx, const dou
 
 extern "C" size_t sglm_xt_vec_workspace_bytes(int32_t C) { return (size_t)sm_count() * 8 * (size_t)std::max(C, 1) * sizeof(double); }
 
-// out[c] = sum_t X[t][c] r[t]: one streaming pass over X (8*T*C bytes), deterministic.
+// out[c] = sum_t X[t][c] r[t]: one streaming pass over X (8*T*C bytes), deterministic.  T = 0 (an empty row slice):
+// X and r may be null, out = 0.
 extern "C" int sglm_xt_vec_f64(const double *X, int64_t ldx, const double *r, int64_t T, int32_t C, double *out,
                                void *workspace, size_t workspace_bytes, void *stream) {
     SGLM_CHECK_ARG(T >= 0 && C > 0 && ldx >= C, SGLM_E_SHAPE, "xt_vec: bad shape");
-    SGLM_CHECK_ARG(X && r && out && workspace, SGLM_E_INVALID_ARG, "xt_vec: null pointer");
+    SGLM_CHECK_ARG((T == 0 || (X && r)) && out && workspace, SGLM_E_INVALID_ARG, "xt_vec: null pointer");
     SGLM_CHECK_ARG(workspace_bytes >= sglm_xt_vec_workspace_bytes(C), SGLM_E_WORKSPACE, "xt_vec: workspace too small");
     cudaStream_t st = (cudaStream_t)stream;
     const int grid = (int)std::max<long long>(1, std::min<long long>((long long)sm_count() * 8, (T + 63) / 64));
