@@ -287,7 +287,8 @@ int sglm_center_stats_f64(const double *A_plus, const double *A_minus, int64_t l
  *   diag(Qc) from sglm_center_stats_f64); prob_yy[p] = yyc
  *   model m uses problem prob_of_model[m] with l1_reg[m] = alpha*l1_ratio*n and
  *   l2_reg[m] = alpha*(1-l1_ratio)*n  (_coordinate_descent.py:781-782).
- *   W[m*ldw + j] is in/out when warm_start != 0, else out (started from 0).
+ *   W[m*ldw + j] is in/out when warm_start & 1, else out (started from 0).  warm_start & 2: at least one sweep (the
+ *   start is never returned on its duality gap alone; the sweep's largest move then decides).
  *   info[m*6 + {0..5}] = {gap, tol*yy, n_iter, n_row_updates, n_blocks_visited, share of time in the register phase}.
  * ------------------------------------------------------------------------- */
 int sglm_enet_cd_gram_f64(const double *const *prob_Q, const double *const *prob_q,
@@ -496,6 +497,17 @@ int sglm_glm_epilogue_f64(double *Eta, int64_t ldb, int32_t n_models, int64_t T,
 int sglm_reduce_parts_f64(const double *parts, int64_t n_elem, int32_t n_parts, double *out, void *stream);
 int sglm_pb_state_words(void);
 int sglm_pb_step_f64(const uint64_t *state_host, const double *const *L_of, void *stream);
+/* Elastic-net models in the batch (l1_ratio[m] = r > 0, l1_ratio [B]; the objective check adds alpha r |w|_1 and the
+ * ridge weight becomes alpha (1 - r)): sglm_pb_step_f64 in which the models enet_models[0 .. n_enet) take a proximal-Newton
+ * step — after the chord solve (which gives their ridge solution for the gap's yy), a warm-started
+ * sglm_enet_cd_gram_f64 solve of  1/2 w'Qw - rhs'w + (alpha r n / hs)|w|_1 + 1/2 (alpha (1 - r) n / hs)|w|^2
+ * replaces their new iterate.  L_of[m] of such a model factors (H~ + alpha (1 - r) n I).  workspace: 16-byte aligned,
+ * sglm_pb_enet_workspace_bytes(C, ldw, n_enet) bytes; info [6 n_enet] = the inner solves' CD info (info[6k + 2]:
+ * sweeps; 0 for a model that took no step).  Arguments are checked before any CUDA call. */
+size_t sglm_pb_enet_workspace_bytes(int32_t C, int64_t ldw, int32_t n_enet);
+int sglm_pb_step_enet_f64(const uint64_t *state_host, const double *const *L_of, const double *l1_ratio,
+                          const int32_t *enet_models, int32_t n_enet, void *workspace, size_t workspace_bytes,
+                          double *info, void *stream);
 
 /* ------------------------------------------------------------------------- *
  * Measurement probe (bench.py; no reference counterpart): reads `n_doubles` doubles

@@ -1297,19 +1297,23 @@ def poisson_irls(Xd, yd, alpha, fit_intercept=True, rw=None, max_iter=100, tol=1
 # (a9, batched) Poisson / Gamma / Tweedie grid: all (fold, alpha) fits advance together (csrc/poisson_batch.cu)
 # --------------------------------------------------------------------------- #
 PB_MAX_BATCH = 256       # models per batch (Eta is T x round_up(B, 64) doubles)
-last_poisson_batch = None    # diagnostics of the most recent batch: iterations, Hessian refreshes, power
+last_poisson_batch = None    # diagnostics of the most recent batch: iterations, Hessian refreshes, power, and for
+                             # elastic-net models their number and the inner CD sweeps summed over models and rounds
 
 
 class PoissonModel:
-    """One fit of a batch: penalty, row-weight vector (index into RW, -1 = all rows), response column, and an optional
-    start point (coef_init [C], intercept_init; default w = 0, b = log mean y)."""
-    __slots__ = ("alpha", "fit_intercept", "rw", "ycol", "max_iter", "tol", "n_tot", "coef_init", "intercept_init")
+    """One fit of a batch: penalty alpha (r |w|_1 + (1 - r)/2 |w|^2) with r = l1_ratio (0: ridge), row-weight vector
+    (index into RW, -1 = all rows), response column, and an optional start point (coef_init [C], intercept_init;
+    default w = 0, b = log mean y)."""
+    __slots__ = ("alpha", "fit_intercept", "rw", "ycol", "max_iter", "tol", "n_tot", "coef_init", "intercept_init",
+                 "l1_ratio")
 
     def __init__(self, alpha, fit_intercept=True, rw=-1, ycol=0, max_iter=100, tol=1e-4, n_tot=None, coef_init=None,
-                 intercept_init=None):
+                 intercept_init=None, l1_ratio=0.0):
         self.alpha, self.fit_intercept, self.rw, self.ycol = float(alpha), bool(fit_intercept), int(rw), int(ycol)
         self.max_iter, self.tol, self.n_tot = int(max_iter), float(tol), n_tot
         self.coef_init, self.intercept_init = coef_init, intercept_init
+        self.l1_ratio = float(l1_ratio)
 
 
 def _loss_name(power):
@@ -1354,7 +1358,9 @@ def poisson_grid_batched(Xd, Yd, models, RW=None):
 def tweedie_grid_batched(Xd, Yd, models, RW=None, power=1.0, comm=None):
     """poisson_grid_batched for the Tweedie family of `power` (1, or > 1; log link): argmin mean(l(y, eta)) +
     alpha/2 |w|^2 with sklearn's HalfTweedieLoss l (p = 2: Gamma, whose Fisher Hessian X' diag(rw) X does not depend
-    on the iterate and is built once per fold).
+    on the iterate and is built once per fold).  A model with l1_ratio r > 0 has the elastic-net penalty
+    alpha r |w|_1 + alpha (1 - r)/2 |w|^2 and takes proximal-Newton steps (sglm_pb_step_enet_f64); it may share a
+    batch with ridge models, whose steps are unchanged.
 
     comm: the rows are sharded over processes — Xd, Yd and RW hold this process's rows, every process calls with the
     same models — and `comm` combines the cross-row reductions: all_reduce(t, op) in place for the integer
@@ -1423,6 +1429,7 @@ def _poisson_batch(Xd, Yd, models, RW, power, comm=None):
     zi = lambda: torch.zeros(B, dtype=torch.int32, device="cuda")
     halv, n_iter, status, flag, has_prev = zi(), zi(), zi(), zi(), zi()
     alpha = _dev([m.alpha for m in models], f64)
+    l1r = _dev([m.l1_ratio for m in models], f64)
     n_tot_d = _dev(n_tot, f64)
     tol = _dev([m.tol for m in models], f64)
     fit_icpt = _dev([int(m.fit_intercept) for m in models], i32)
@@ -1464,7 +1471,8 @@ def _poisson_batch(Xd, Yd, models, RW, power, comm=None):
         rw_vec = RW[rw] if rw >= 0 else None
         hess, h11 = _pb_hessian(Xd, ycontig[models[ref].ycol], rw_vec, W[ref], b[ref:ref + 1], fi, float(n_tot[ref]), use_tc,
                                 power, comm)
-        an = _dev([models[i].alpha * n_tot[i] for i in idxs], f64)
+        an = _dev([models[i].alpha * n_tot[i] if models[i].l1_ratio == 0 else
+                   models[i].alpha * (1.0 - models[i].l1_ratio) * n_tot[i] for i in idxs], f64)
         wb = nat.lib().sglm_ridge_workspace_bytes(C, hess.ldq, len(idxs))
         work = torch.empty(wb // 8, dtype=torch.float64, device="cuda")
         Wtmp = _empty((len(idxs), ldw))
@@ -1496,8 +1504,8 @@ def _poisson_batch(Xd, Yd, models, RW, power, comm=None):
         if rw < 0 or (-1, fi) not in groups:
             continue
         g0 = gkeys.index((-1, fi))
-        by_alpha = {(models[i].alpha, models[i].ycol == 0): i for i in groups[gkeys[g0]]}
-        pairs = [(i, by_alpha.get((models[i].alpha, True))) for i in groups[gkeys[g]]]
+        by_alpha = {(models[i].alpha, models[i].l1_ratio, models[i].ycol == 0): i for i in groups[gkeys[g0]]}
+        pairs = [(i, by_alpha.get((models[i].alpha, models[i].l1_ratio, True))) for i in groups[gkeys[g]]]
         if all(j is not None and models[i].coef_init is None and models[j].coef_init is None for i, j in pairs):
             borrowed[g] = (g0, pairs)
     for g in range(n_h):
@@ -1526,6 +1534,13 @@ def _poisson_batch(Xd, Yd, models, RW, power, comm=None):
     state = np.array(words, dtype=np.uint64)
     state_p = state.ctypes.data_as(ctypes.c_void_p)
     RWp, ldrw = (ptr(RW), RW.stride(0)) if RW is not None else (None, 0)
+    enet = [i for i, m in enumerate(models) if m.l1_ratio != 0]
+    if enet:
+        enet_idx = _dev(enet, i32)
+        en_bytes = nat.lib().sglm_pb_enet_workspace_bytes(C, ldw, len(enet))
+        en_ws = torch.empty(en_bytes // 8 + 1, dtype=torch.float64, device="cuda")
+        en_info = _zeros((len(enet), 6))
+        sweeps = torch.zeros((), dtype=torch.float64, device="cuda")
     it = 0
     max_rounds = int(max(m.max_iter for m in models)) + 40
     while it < max_rounds:
@@ -1537,7 +1552,12 @@ def _poisson_batch(Xd, Yd, models, RW, power, comm=None):
              stream_ptr())
         if comm is not None:
             red.copy_(comm.combine(red))
-        call("sglm_pb_step_f64", state_p, ptr(L_of), stream_ptr())
+        if enet:
+            call("sglm_pb_step_enet_f64", state_p, ptr(L_of), ptr(l1r), ptr(enet_idx), len(enet), ptr(en_ws), en_ws.numel() * 8,
+                 ptr(en_info), stream_ptr())
+            sweeps += en_info[:, 2].sum()
+        else:
+            call("sglm_pb_step_f64", state_p, ptr(L_of), stream_ptr())
         it += 1
         host = torch.stack([status.to(torch.float64), step_out, ratio_out]).cpu().numpy()     # the one read-back per iteration
         st_h, step_h, ratio_h = host[0], host[1], host[2]
@@ -1562,9 +1582,11 @@ def _poisson_batch(Xd, Yd, models, RW, power, comm=None):
     n_it = n_iter.cpu().numpy().astype(np.int64)
     st_f = status.cpu().numpy().astype(np.int64)
     st_f[st_f == 0] = 2
-    return W[:, :C].contiguous(), b.clone(), n_it, st_f, dict(rounds=it, refreshes=dict(n_refresh), models=B,
-                                                              hessian_groups=n_h, tensor_core_hessian=bool(use_tc),
-                                                              power=power)
+    diag = dict(rounds=it, refreshes=dict(n_refresh), models=B, hessian_groups=n_h, tensor_core_hessian=bool(use_tc),
+                power=power)
+    if enet:
+        diag.update(enet_models=len(enet), inner_sweeps=int(sweeps.item()))
+    return W[:, :C].contiguous(), b.clone(), n_it, st_f, diag
 
 
 def poisson_scores_batched(Xd, Yd, W, b, ycol, rw_a, rw_b, RW):

@@ -1,7 +1,8 @@
 """
 Estimator objects behind `GLM.model` — the GPU counterparts of the scikit-learn classes
 the reference instantiates (backend/sglm.py:2, :95-130): LinearRegression, Ridge, Lasso,
-ElasticNet, TweedieRegressor (power 1 = Poisson, 2 = Gamma, any power > 1; log link).  Same constructor keywords (unknown keywords raise
+ElasticNet, TweedieRegressor (power 1 = Poisson, 2 = Gamma, any power > 1; log link), plus TweedieElasticNet
+(the same families with an L1 + L2 penalty; no scikit-learn counterpart).  Same constructor keywords (unknown keywords raise
 TypeError exactly as scikit-learn does, which is how stale kwargs such as `reg_lambda`
 fail in the reference), same fitted attributes (`coef_`, `intercept_`, `n_iter_`,
 `dual_gap_`), same `fit / predict / score`.  All arithmetic runs in libsglm_b200.so.
@@ -241,3 +242,56 @@ class TweedieRegressor(_Base):
         self._check_y(yd)
         s, _ = eng.score_sums(Xd, yd, self.coef_, self.intercept_, power=self.power)
         return eng.tweedie_d2_from_sums(s, self.power)
+
+
+class TweedieElasticNet(_Base):
+    """Tweedie GLM with log link and an elastic-net penalty — an extension with no scikit-learn counterpart:
+
+        argmin  mean(l(y, eta)) + alpha l1_ratio |w|_1 + alpha (1 - l1_ratio)/2 |w|^2,   eta = X w + b (b unpenalised)
+
+    with sklearn's HalfTweedieLoss l of `power` (1 = Poisson, 2 = Gamma, any power > 1), the L1 term scaled by the
+    mean loss as in glmnet / pyglmnet and this project's ElasticNet.  At l1_ratio = 0 this is TweedieRegressor's
+    objective.  Fitted by the batched solver with one model for every power (proximal-Newton steps: the quadratic
+    model of the chord step solved by Gram coordinate descent); `score` is the family's D^2."""
+    _link = 1
+    kind = "tweedie_enet"
+
+    def __init__(self, *, power=0.0, alpha=1.0, l1_ratio=0.5, fit_intercept=True, link="auto", max_iter=100,
+                 tol=1e-4, warm_start=False):
+        self.power, self.alpha, self.l1_ratio, self.fit_intercept, self.link = power, alpha, l1_ratio, fit_intercept, link
+        self.max_iter, self.tol, self.warm_start = max_iter, tol, warm_start
+        self._check_params()
+        self._check_family()
+
+    _check_family = TweedieRegressor._check_family
+    _check_y = TweedieRegressor._check_y
+    score = TweedieRegressor.score
+
+    def _check_params(self):
+        if not (0.0 <= self.l1_ratio <= 1.0):
+            raise ValueError(f"The 'l1_ratio' parameter of TweedieElasticNet must be a float in the range [0.0, 1.0]; "
+                             f"got {self.l1_ratio!r}.")
+        if not (self.alpha >= 0.0):
+            raise ValueError(f"The 'alpha' parameter of TweedieElasticNet must be a float in the range [0.0, inf); "
+                             f"got {self.alpha!r}.")
+
+    def fit(self, X, y, sample_weight=None):
+        if sample_weight is not None:
+            raise NotImplementedError("sample_weight is never passed by the reference")
+        self._check_params()
+        self._check_family()
+        Xd, yd = eng.device_matrix(X), eng.device_vector(y)
+        import torch
+        self._check_y(yd)
+        if not bool(torch.isfinite(Xd).all().item()):
+            raise ValueError("Input X contains NaN or infinity.")
+        ci = getattr(self, "coef_", None) if self.warm_start else None
+        ii = getattr(self, "intercept_", None) if self.warm_start else None
+        m = eng.PoissonModel(self.alpha, self.fit_intercept, max_iter=self.max_iter, tol=self.tol, coef_init=ci,
+                             intercept_init=ii, l1_ratio=self.l1_ratio)
+        W, b, n_it, _ = eng.tweedie_grid_batched(Xd, yd[:, None], [m], None, float(self.power))
+        self.coef_ = W[0].cpu().numpy()
+        self.intercept_ = float(b[0].item()) if self.fit_intercept else 0.0
+        self.n_iter_ = int(n_it[0])
+        self.n_features_in_ = Xd.shape[1]
+        return self

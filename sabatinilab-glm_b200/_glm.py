@@ -14,6 +14,11 @@ Deliberate deviations (crash / hang fixes, documented in DESIGN.md):
   * Gamma / Tweedie: the GPU path fits power 1 and any power > 1 with log link; power <= 0,
     0 < power < 1 and link='identity' raise NotImplementedError.  With all-zero y and
     1 < power < 2 the fit raises ValueError (scikit-learn returns an intercept of -inf).
+  * Poisson / Gamma / Tweedie with `l1_ratio` (an extension: the reference's TweedieRegressor has no
+    such keyword and raises TypeError): with l1_ratio and alpha both non-zero the model is a
+    TweedieElasticNet, mean loss + alpha (l1_ratio |w|_1 + (1 - l1_ratio)/2 |w|^2) as in pyglmnet,
+    which the reference's users fitted before; l1_ratio == 0 or alpha == 0 drops the keyword and
+    builds TweedieRegressor, as l1_ratio == 0 builds Ridge for the Gaussian family.
   * Logistic / Multinomial are outside the hot-path scope (SURVEY.md §8) and raise
     NotImplementedError.
 """
@@ -23,7 +28,7 @@ import numpy as np
 
 import _engine as eng
 from _estimators import (ConvergenceWarning, ElasticNet, Lasso, LinearRegression, Ridge,  # noqa: F401
-                         TweedieRegressor)
+                         TweedieElasticNet, TweedieRegressor)
 
 
 class NotYetImplementedError(NameError, NotImplementedError):
@@ -68,11 +73,15 @@ class GLM():
                 Base = Lasso
             else:
                 Base = ElasticNet
-        elif model_name in {'Poisson', 'Gamma'}:
-            kwargs['power'] = self.tweedie_lookup[model_name]
+        elif model_name in {'Poisson', 'Gamma', 'Tweedie'}:
+            if model_name != 'Tweedie':
+                kwargs['power'] = self.tweedie_lookup[model_name]
             Base = TweedieRegressor
-        elif model_name in {'Tweedie'}:
-            Base = TweedieRegressor
+            if 'l1_ratio' in kwargs:
+                if kwargs['l1_ratio'] == 0 or kwargs.get('alpha', 1.0) == 0:
+                    del kwargs['l1_ratio']
+                else:
+                    Base = TweedieElasticNet
         elif model_name in {'Logistic', 'Multinomial'}:
             raise NotImplementedError("Logistic/Multinomial GLMs are outside the B200 hot-path scope")
         elif model_name in {'PCA Normal', 'PCA Gaussian'}:

@@ -100,6 +100,8 @@ _PROTOTYPES = {
                                      c_i32, c_vp, c_vp, c_sz, c_vp]),
     "sglm_pb_state_words": (c_i32, []),
     "sglm_pb_step_f64": (c_i32, [c_vp, c_vp, c_vp]),
+    "sglm_pb_enet_workspace_bytes": (c_sz, [c_i32, c_i64, c_i32]),
+    "sglm_pb_step_enet_f64": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_sz, c_vp, c_vp]),
     "sglm_col_moments_workspace_bytes": (c_sz, [c_i64, c_i32]),
     "sglm_col_moments_f64": (c_i32, [c_vp, c_i64, c_i64, c_i32, c_i32, c_i32, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "sglm_zscore_apply_f64": (c_i32, [c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_vp, c_i64, c_vp]),
@@ -173,7 +175,7 @@ _KERNELS_PER_CALL = {"sglm_suffstats_f64": 3, "sglm_gram_tc_analyze_f64": 2, "sg
                      "sglm_gram_tc_analyze_scaled_f64": 2, "sglm_quadform_gemm_f64": 3, "sglm_xt_vec_f64": 2, "sglm_score_f64": 2,
                      "sglm_poisson_irls_prepare_f64": 2, "sglm_timeshift_f64": 2, "sglm_pb_xt_r_f64": 2, "sglm_pb_epilogue_f64": 2,
                      "sglm_glm_epilogue_f64": 2, "sglm_score_glm_f64": 2, "sglm_glm_irls_prepare_f64": 2,
-                     "sglm_pb_step_f64": 3, "sglm_lag_valid_rows": 3, "sglm_col_moments_f64": 4, "sglm_mask_compact_rows": 3}
+                     "sglm_pb_step_f64": 3, "sglm_pb_step_enet_f64": 6, "sglm_lag_valid_rows": 3, "sglm_col_moments_f64": 4, "sglm_mask_compact_rows": 3}
 _timing = None         # when enabled: list of (name, start_event, end_event) on the current stream
 
 

@@ -322,19 +322,24 @@ __device__ __forceinline__ double pb_block_max(double v, double *sh) {
     return s;
 }
 
-// objective check / step halving, else the right-hand side of the chord step  (H~ + a n I) w_new = H~ w - g
+// objective check / step halving, else the right-hand side of the chord step  (H~ + a n I) w_new = H~ w - g.
+// l1_ratio [B] (null: all 0): the penalty is alpha r |w|_1 + alpha (1 - r)/2 |w|^2
 __global__ void __launch_bounds__(256)
-pb_rhs_kernel(PbState s) {
+pb_rhs_kernel(PbState s, const double *__restrict__ l1_ratio) {
     __shared__ double sh[8];
     extern __shared__ __align__(16) double wsh[];          // [C] current w
     const int m = blockIdx.x, tid = threadIdx.x;
     if (s.status[m] != 0) { if (tid == 0) s.flag[m] = 0; return; }
     double *w = s.W + (long long)m * s.ldw;
     const double *wp = s.Wprev + (long long)m * s.ldw;
-    double ww = 0.0;
-    for (int j = tid; j < s.C; j += 256) { const double v = w[j]; wsh[j] = v; ww = fma(v, v, ww); }
+    double ww = 0.0, w1 = 0.0;
+    for (int j = tid; j < s.C; j += 256) { const double v = w[j]; wsh[j] = v; ww = fma(v, v, ww); w1 += fabs(v); }
     ww = pb_block_sum(ww, sh);
-    const double f = s.sums[4 * m + 0] / s.n_tot[m] + 0.5 * s.alpha[m] * ww;
+    w1 = pb_block_sum(w1, sh);
+    const double r1 = l1_ratio ? l1_ratio[m] : 0.0;
+    // r = 0: alpha (1 - 0) = alpha and no L1 term, so f (and every halving decision) has the bits of the ridge path
+    double f = s.sums[4 * m + 0] / s.n_tot[m] + 0.5 * (s.alpha[m] * (1.0 - r1)) * ww;
+    if (r1 != 0.0) f += s.alpha[m] * r1 * w1;
     const double fp = s.fprev[m];
     const bool worse = s.has_prev[m] && !(f <= fp + 1e-12 * fmax(1.0, fabs(fp)));
     if (worse && s.halv[m] < 30) {
@@ -361,6 +366,83 @@ pb_rhs_kernel(PbState s) {
         if (lane == 0) rhs[j] = d + (-s.Gw[(long long)j * s.ldb + m] + (icpt ? xbar[j] * g_b : 0.0)) * inv_hs;
     }
     if (tid == 0) { s.halv[m] = 0; s.fcur[m] = f; s.flag[m] = 1; }
+}
+
+// ---- elastic-net models (l1_ratio > 0): proximal-Newton step.  The quadratic model of the chord step keeps its
+// Hessian and right-hand side; the triangular solves are replaced by a warm-started Gram coordinate-descent solve of
+//   min_w 1/2 w'Qw - rhs'w + l1 |w|_1 + l2/2 |w|^2,   l1 = alpha r n / hs,  l2 = alpha (1 - r) n / hs
+// (enet_cd_gram_kernel, solvers.cu).  Its duality gap needs a yy consistent with (Q, rhs): yy = rhs'(Q + l2 I)^-1 rhs,
+// the ridge solution coming from the model's cached factor of (Q + alpha (1 - r) n I) (the chord solve that precedes
+// this kernel), so that R^2 + l2 |w|^2 = (w - w_ridge)'(Q + l2 I)(w - w_ridge) >= 0.  A fold's first step borrows
+// the full-data factor (hs != 1); there yy belongs to a nearby l2 and only makes that one step's stopping test
+// approximate: the later steps use the fold's own Hessian (hs = 1).
+//
+// Inner tolerance: the kernel stops after a sweep that moved no coordinate by more than tol * max|w| and whose gap is
+// <= tol * yy.  The sweep test is what resolves a small step: the gap is a difference of terms of size
+// yy = |w_ridge|^2_(Q + l2 I) (rounding ~1e-16 yy), so it only bounds a step d through |d|_(Q + l2 I) <= sqrt(2 gap),
+// i.e. to ~1e-8 relative.  Hence the solve is started with "at least one sweep" (a start whose gap is below tol * yy
+// would otherwise be returned untouched and end the outer iteration up to ~1e-7 from its fixed point), and tol = 1e-13:
+// the inner error (~1e-13 |w| times the CD contraction factor) stays far below what the outer rule
+// (step * rho / (1 - rho) <= min(tol, 1e-8)) resolves, so inexact inner solves neither stall nor end the outer iteration,
+// while the gap test at tol * yy = 1e-13 yy stays well above its rounding floor.
+constexpr double PB_ENET_TOL = 1e-13;
+// sweeps per inner solve: a cap, not a budget — a warm start near the optimum needs a few
+constexpr int PB_ENET_SWEEPS = 1000;
+
+// workspace of sglm_pb_step_enet_f64 (n_enet models): W [n][ldw], diag [n][ldw], yy / l1 / l2 / tol [n],
+// Q / q / diag pointers [n], max_iter / problem ids [n] (int32)
+struct PbEnetWork {
+    double *W, *dg, *yy, *l1, *l2, *tol;
+    const double **pQ, **pq, **pd;
+    int *max_iter, *pid;
+};
+__host__ __device__ inline PbEnetWork pb_enet_carve(void *ws, long long ldw, int n) {
+    PbEnetWork e;
+    double *d = (double *)ws;
+    e.W = d; d += (long long)n * ldw;
+    e.dg = d; d += (long long)n * ldw;
+    e.yy = d; d += n; e.l1 = d; d += n; e.l2 = d; d += n; e.tol = d; d += n;
+    e.pQ = (const double **)d; d += n; e.pq = (const double **)d; d += n; e.pd = (const double **)d; d += n;
+    e.max_iter = (int *)d; e.pid = e.max_iter + n;
+    return e;
+}
+
+// one CTA per elastic-net model k (model m = idx[k]): the inner problem.  Models without a step this round (flag != 1:
+// halving, converged, max_iter) get w = 0 and max_iter 0: the solve returns at once and its result is not used.
+__global__ void __launch_bounds__(256)
+pb_enet_prep_kernel(PbState s, const double *__restrict__ l1_ratio, const int *__restrict__ idx, PbEnetWork e) {
+    __shared__ double sh[8];
+    const int k = blockIdx.x, tid = threadIdx.x, m = idx[k];
+    const bool step = s.flag[m] == 1;
+    const int h = s.hess_id[m];
+    const double *Q = s.HQ[h];
+    const double *q = s.rhs + (long long)m * s.ldw, *wr = s.Wnew + (long long)m * s.ldw, *w = s.W + (long long)m * s.ldw;
+    double *wk = e.W + (long long)k * s.ldw, *dk = e.dg + (long long)k * s.ldw;
+    double yy = 0.0;
+    for (int j = tid; j < s.C; j += 256) {
+        dk[j] = Q[(long long)j * s.ldq + j];
+        wk[j] = step ? w[j] : 0.0;
+        yy = fma(q[j], wr[j], yy);
+    }
+    yy = pb_block_sum(yy, sh);
+    if (tid == 0) {
+        const double r1 = l1_ratio[m], an = s.alpha[m] * s.n_tot[m] / s.hscale[m];
+        e.pQ[k] = Q; e.pq[k] = q; e.pd[k] = dk;
+        e.yy[k] = yy;
+        e.l1[k] = an * r1;
+        e.l2[k] = an * (1.0 - r1);
+        e.tol[k] = PB_ENET_TOL;
+        e.max_iter[k] = step ? PB_ENET_SWEEPS : 0;
+        e.pid[k] = k;
+    }
+}
+
+// the inner solutions become the models' new iterates
+__global__ void __launch_bounds__(256)
+pb_enet_scatter_kernel(PbState s, const int *__restrict__ idx, PbEnetWork e) {
+    const int k = blockIdx.x, m = idx[k];
+    if (s.flag[m] != 1) return;
+    for (int j = threadIdx.x; j < s.C; j += 256) s.Wnew[(long long)m * s.ldw + j] = e.W[(long long)k * s.ldw + j];
 }
 
 // intercept, step size, convergence
@@ -592,6 +674,13 @@ extern "C" int sglm_chol_solve_batched_f64(const double *const *L_of, int64_t ld
                                            double *out, int64_t ld, const int32_t *flags, int32_t n_systems,
                                            void *stream);
 
+extern "C" int sglm_enet_cd_gram_f64(const double *const *prob_Q, const double *const *prob_q,
+                                     const double *const *prob_diag, const double *prob_yy, int64_t ldq, int32_t C,
+                                     const int32_t *prob_of_model, const double *l1_reg, const double *l2_reg,
+                                     const double *tol, const int32_t *max_iter, int32_t n_models, int32_t warm_start,
+                                     int32_t do_screening, double *W, int64_t ldw, double *info, void *stream);
+namespace sglm { size_t enet_cd_smem_bytes(int C); }
+
 extern "C" int sglm_pb_step_f64(const uint64_t *state_host, const double *const *L_of, void *stream) {
     SGLM_CHECK_ARG(state_host && L_of, SGLM_E_INVALID_ARG, "pb_step: null pointer");
     static_assert(sizeof(PbState) % 8 == 0, "PbState is passed as 64-bit words");
@@ -602,10 +691,58 @@ extern "C" int sglm_pb_step_f64(const uint64_t *state_host, const double *const 
     const size_t smem = (size_t)s.C * sizeof(double);
     SGLM_CHECK_ARG(smem <= 200 * 1024, SGLM_E_UNSUPPORTED, "pb_step: C=%d too large", s.C);
     SGLM_CUDA_OK(cudaFuncSetAttribute(pb_rhs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    pb_rhs_kernel<<<s.B, 256, smem, st>>>(s);
+    pb_rhs_kernel<<<s.B, 256, smem, st>>>(s, nullptr);
     SGLM_LAUNCH_OK("pb_rhs_kernel");
     const int rc = sglm_chol_solve_batched_f64(L_of, s.ldq, s.C, s.rhs, s.Wnew, s.ldw, s.flag, s.B, stream);
     if (rc != SGLM_OK) return rc;
+    pb_finish_kernel<<<s.B, 256, 0, st>>>(s);
+    SGLM_LAUNCH_OK("pb_finish_kernel");
+    return SGLM_OK;
+}
+
+extern "C" size_t sglm_pb_enet_workspace_bytes(int32_t C, int64_t ldw, int32_t n_enet) {
+    if (C <= 0 || ldw < C || n_enet <= 0) return 0;
+    return (size_t)n_enet * (size_t)(2 * ldw + 8) * sizeof(double);
+}
+
+// sglm_pb_step_f64 for a batch with elastic-net models (l1_ratio [B]: r of every model, 0 for a ridge model): the
+// models enet_models[0 .. n_enet) (those with r > 0, distinct) take a proximal-Newton step — the chord step's right-hand side, then a warm-started Gram CD solve of the
+// quadratic model with the L1 term (enet_cd_gram_kernel) instead of the triangular solves; the others take the chord
+// step.  L_of[m] of an elastic-net model is its factor of (H~ + alpha (1 - r) n I).  info [6 n_enet]: the inner
+// solves' sglm_enet_cd_gram_f64 info (info[6k + 2] = sweeps).
+extern "C" int sglm_pb_step_enet_f64(const uint64_t *state_host, const double *const *L_of, const double *l1_ratio,
+                                     const int32_t *enet_models, int32_t n_enet, void *workspace,
+                                     size_t workspace_bytes, double *info, void *stream) {
+    SGLM_CHECK_ARG(state_host && L_of, SGLM_E_INVALID_ARG, "pb_step_enet: null pointer");
+    PbState s;
+    memcpy(&s, state_host, sizeof(PbState));
+    SGLM_CHECK_ARG(s.C > 0 && s.B > 0 && s.ldw >= s.C && s.ldq >= s.C && s.ldb >= s.B, SGLM_E_SHAPE,
+                   "pb_step_enet: bad shape");
+    SGLM_CHECK_ARG(n_enet >= 1 && n_enet <= s.B, SGLM_E_SHAPE, "pb_step_enet: n_enet=%d outside [1, B=%d]", n_enet, s.B);
+    SGLM_CHECK_ARG(l1_ratio && enet_models && workspace && info, SGLM_E_INVALID_ARG, "pb_step_enet: null pointer");
+    SGLM_CHECK_ARG(((uintptr_t)workspace & 15) == 0, SGLM_E_ALIGN, "pb_step_enet: 16-byte alignment");
+    SGLM_CHECK_ARG(workspace_bytes >= sglm_pb_enet_workspace_bytes(s.C, s.ldw, n_enet), SGLM_E_WORKSPACE,
+                   "pb_step_enet: workspace too small");
+    const size_t smem = (size_t)s.C * sizeof(double);
+    SGLM_CHECK_ARG(smem <= 200 * 1024 && enet_cd_smem_bytes(s.C) <= 227 * 1024, SGLM_E_UNSUPPORTED,
+                   "pb_step_enet: C=%d too large", s.C);
+    cudaStream_t st = (cudaStream_t)stream;
+    SGLM_CUDA_OK(cudaFuncSetAttribute(pb_rhs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    pb_rhs_kernel<<<s.B, 256, smem, st>>>(s, l1_ratio);
+    SGLM_LAUNCH_OK("pb_rhs_kernel");
+    // every stepping model's chord solve: the new iterate of a ridge model, w_ridge (for yy) of an elastic-net model
+    int rc = sglm_chol_solve_batched_f64(L_of, s.ldq, s.C, s.rhs, s.Wnew, s.ldw, s.flag, s.B, stream);
+    if (rc != SGLM_OK) return rc;
+    const PbEnetWork e = pb_enet_carve(workspace, s.ldw, n_enet);
+    pb_enet_prep_kernel<<<n_enet, 256, 0, st>>>(s, l1_ratio, enet_models, e);
+    SGLM_LAUNCH_OK("pb_enet_prep_kernel");
+    // no screening: a yy from a borrowed factor (first step of a fold) is not a certified bound
+    // warm start (bit 0) with at least one sweep (bit 1)
+    rc = sglm_enet_cd_gram_f64(e.pQ, e.pq, e.pd, e.yy, s.ldq, s.C, e.pid, e.l1, e.l2, e.tol, e.max_iter, n_enet, 3, 0,
+                               e.W, s.ldw, info, stream);
+    if (rc != SGLM_OK) return rc;
+    pb_enet_scatter_kernel<<<n_enet, 256, 0, st>>>(s, enet_models, e);
+    SGLM_LAUNCH_OK("pb_enet_scatter_kernel");
     pb_finish_kernel<<<s.B, 256, 0, st>>>(s);
     SGLM_LAUNCH_OK("pb_finish_kernel");
     return SGLM_OK;

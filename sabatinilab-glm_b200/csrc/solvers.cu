@@ -156,6 +156,9 @@ enet_cd_gram_kernel(const double *const *__restrict__ prob_Q, const double *cons
     const bool is_seq = warp == 0;
     const bool screening = do_screening && (l1 != 0.0);
     const int dbg_sel = warm_start >> 8;      // diagnostics: what info[6m+5] reports (6: start time, 7: duration, ns)
+    // bit 1: at least one sweep — the start is not returned on its duality gap alone (the gap, a difference of terms of
+    // size yy, cannot resolve a step below ~1e-8 |w|: a warm start at an outer iterate needs the sweep test to decide)
+    const bool sweep_once = (warm_start & 2) != 0;
     warm_start &= 1;
     const unsigned long long gt_begin = global_timer_ns();
 
@@ -259,7 +262,7 @@ enet_cd_gram_kernel(const double *const *__restrict__ prob_Q, const double *cons
             }
         }
         gap = compute_gap();
-        done = (gap >= 0.0 && gap <= tol) || max_iter <= 0;
+        done = (!sweep_once && gap >= 0.0 && gap <= tol) || max_iter <= 0;
         if (!done && screening) screen(true);
         if (lane == 0) ctl[1] = done ? 1u : 0u;
     }
@@ -1006,7 +1009,8 @@ extern "C" int sglm_center_stats_f64(const double *A_plus, const double *A_minus
     return SGLM_OK;
 }
 
-static size_t cd_smem_bytes(int C) {
+namespace sglm { size_t enet_cd_smem_bytes(int C); }
+size_t sglm::enet_cd_smem_bytes(int C) {
     const int Cp = (C + 1) & ~1, nblk = (C + 31) / 32;
     return (size_t)(2 * Cp + 2 * 1024 + 128 + 32) * sizeof(double) + (size_t)(2 * nblk + 2) * sizeof(unsigned) + (size_t)nblk + 64;
 }
@@ -1021,7 +1025,7 @@ extern "C" int sglm_enet_cd_gram_f64(const double *const *prob_Q, const double *
     if (n_models == 0) return SGLM_OK;
     SGLM_CHECK_ARG(prob_Q && prob_q && prob_diag && prob_yy && prob_of_model && l1_reg && l2_reg && tol && max_iter && W && info,
                    SGLM_E_INVALID_ARG, "enet_cd: null pointer");
-    const size_t smem = cd_smem_bytes(C);
+    const size_t smem = enet_cd_smem_bytes(C);
     SGLM_CHECK_ARG(smem <= 227 * 1024, SGLM_E_UNSUPPORTED,
                    "enet_cd: C=%d needs %zu bytes of shared memory per model (> 227 KB)", C, smem);
     cudaStream_t st = (cudaStream_t)stream;

@@ -527,11 +527,13 @@ def _tweedie_cv(Xd, Yd, ycol_of_roll, RW, F, glms, rolls, score_method, power, c
     for glm, r in zip(glms, rolls):
         est = glm.model
         est._check_family()
+        l1_ratio = est.l1_ratio if est.kind == "tweedie_enet" else 0.0
         for f in range(F):
             models.append(eng.PoissonModel(est.alpha, est.fit_intercept, rw=f, ycol=ycol_of_roll[r],
-                                           max_iter=est.max_iter, tol=est.tol))
+                                           max_iter=est.max_iter, tol=est.tol, l1_ratio=l1_ratio))
             ycol.append(ycol_of_roll[r]); rw_a.append(f); rw_b.append(F + f)
-        models.append(eng.PoissonModel(est.alpha, est.fit_intercept, rw=-1, ycol=0, max_iter=est.max_iter, tol=est.tol))
+        models.append(eng.PoissonModel(est.alpha, est.fit_intercept, rw=-1, ycol=0, max_iter=est.max_iter, tol=est.tol,
+                                       l1_ratio=l1_ratio))
         ycol.append(0); rw_a.append(-1); rw_b.append(-2)          # the refit uses the UN-rolled y (backend/sglm_cv.py:181)
     Wd, bd, n_it, status = eng.tweedie_grid_batched(Xd, Yd, models, RW, power, comm)
     sums = eng.tweedie_scores_batched(Xd, Yd, Wd, bd, ycol, rw_a, rw_b, RW, power, comm)
@@ -583,10 +585,11 @@ def _cv_batch(X, y, cv_idx, entries, beta_, beta0_, score_method):
         glms.append(sglm_.GLM(model_name, beta0_=beta0_, beta_=beta_, **kw))   # refit object (:180)
     out = [None] * len(entries)
     gauss = [i for i, g in enumerate(glms) if g.model.kind in ("ols", "ridge", "lasso", "enet")]
-    # the log-link families: one batch per distinct power, Poisson (power 1) first
+    # the log-link families: one batch per distinct power, Poisson (power 1) first; elastic-net sets join the batch of
+    # their power
     by_power = {}
     for i, g in enumerate(glms):
-        if g.model.kind in ("poisson", "tweedie"):
+        if g.model.kind in ("poisson", "tweedie", "tweedie_enet"):
             by_power.setdefault(1.0 if g.model.kind == "poisson" else g.model.power, []).append(i)
     if gauss:
         res = _gaussian_grid(Xd, yd, cv_idx, [glms[i] for i in gauss], [rolls[i] for i in gauss], score_method)

@@ -226,7 +226,7 @@ class RankComm:
         return eng.reduce_parts(parts, self.world).reshape(t.shape)
 
 
-LOG_LINK_KINDS = ("poisson", "tweedie")
+LOG_LINK_KINDS = ("poisson", "tweedie", "tweedie_enet")
 GAUSSIAN_KINDS = ("ols", "ridge", "lasso", "enet")
 
 
@@ -248,6 +248,8 @@ def cv_grid_strong(X0, shift_amt_list, y, cv_idx, model_name, glm_kwarg_lst, ver
     sums, X'R, the weighted Hessian Gram, the scores) is combined over the ranks (RankComm), so every rank runs every
     log-link model in lock step and holds all their coefficients.  Unlike the Gaussian statistics, the fp64 gradient
     sums are re-associated over the ranks: the log-link results agree with the one-GPU grid to rounding, not to the bit.
+
+    Sets with an l1_ratio (TweedieElasticNet) run in the batch of their power, with the same combined sums.
 
     rows = (lo, hi): base rows kept after `dropna` (default: the rows without NaN padding).  Folds must be the
     usual complement pairs with duplicate-free test rows (cv_idx_by_*); Gaussian, Poisson, Gamma and Tweedie

@@ -1,11 +1,12 @@
 """The other BASELINE.json configurations on one B200, each with the reference's CPU path timed beside it
 (SURVEY.md §8d): configs[0] single ElasticNet fit 100k x 410, configs[1] Ridge CV 5 folds x 20 alphas 500k x 1220,
 configs[3] Poisson alpha sweep 20 alphas x 5 folds (+ refits) 1M x 800, and the same sweep for the Gamma family (c4g)
-and the Tweedie family with power 1.5 (c4t) on a response of that family.  One JSON line per configuration:
+and the Tweedie family with power 1.5 (c4t) on a response of that family, and the Poisson sweep with elastic-net
+penalties (c4en: 20 alphas x l1_ratio 0.1 / 0.5 / 0.9 x (5 folds + refit) = 360 fits).  One JSON line per configuration:
 device-resident time (CUDA events, warm-up excluded), end-to-end time from host numpy arrays, per-entry-point
 milliseconds, and the CPU baseline (scikit-learn through the oracle port, bounded sample, extrapolated and labelled).
 
-    python scripts/config_bench.py [c1] [c2] [c4] [c4g] [c4t] [--no-cpu]     (default: c1 c2 c4)
+    python scripts/config_bench.py [c1] [c2] [c4] [c4g] [c4t] [c4en] [--no-cpu]     (default: c1 c2 c4)
 """
 import json
 import os
@@ -220,11 +221,37 @@ def run_c4_family(name, model_name, power):
             "per_entry_ms": per}
 
 
+def run_c4en(cpu):
+    """c4 (Poisson response, design, folds) with elastic-net sets: no CPU baseline (scikit-learn has no L1 Poisson)."""
+    X0_h, X0, shifts, (lo, hi), y, n = session(1_000_000, 20, -20, 19, 4, poisson=True)
+    folds_h = synth_data.synth_folds(n, 5, 4)
+    folds = [(torch.from_numpy(a).cuda(), torch.from_numpy(b).cuda()) for a, b in folds_h]
+    grid = [dict(alpha=float(a), l1_ratio=r, model_name="Poisson") for r in (0.1, 0.5, 0.9) for a in np.logspace(-4, 1, 20)]
+
+    def dev():
+        d = sglm_pp.timeshift_multiple(X0, shift_amt_list=shifts)[lo:hi]
+        return sglm_cv.cv_glm_mult_params(d, y, folds, "Poisson", [dict(g) for g in grid], score_method="r2")
+    sec, r, per = timed(dev, reps=2, warm=1)
+    diag = _engine.last_poisson_batch or []
+    nnz = [int(np.count_nonzero(x["model"].coef_)) for x in r["full_cv_results"]]
+    return {"config": "c4en: Poisson GLM (log link, elastic net) alpha sweep logspace(-4, 1, 20) x l1_ratio 0.1 / 0.5 / 0.9 x "
+                      "(5 folds + refit) = 360 fits in batches of %d, 1M timepoints x 20 predictors x 40 shifts = 800 columns, "
+                      "every fit driven to its optimum (step bound 1e-8)" % _engine.PB_MAX_BATCH,
+            "fits": 360, "seconds": sec, "fits_per_s": 360 / sec, "best_params": r["best_params"], "batch": diag,
+            "rounds": [d["rounds"] for d in diag], "refreshes": [d["refreshes"] for d in diag],
+            "inner_cd_sweeps": [d.get("inner_sweeps") for d in diag],
+            "refit_nonzero_min_max": [min(nnz), max(nnz)],
+            "n_iter_min_max": [int(min(np.min(x["_fit_info"]["n_iter"]) for x in r["full_cv_results"])),
+                               int(max(np.max(x["_fit_info"]["n_iter"]) for x in r["full_cv_results"]))],
+            "per_entry_ms": per}
+
+
 if __name__ == "__main__":
     which = [a for a in sys.argv[1:] if not a.startswith("--")] or ["c1", "c2", "c4"]
     cpu = "--no-cpu" not in sys.argv
     runs = {"c1": run_c1, "c2": run_c2, "c4": run_c4,
-            "c4g": lambda cpu: run_c4_family("c4g", "Gamma", 2.0), "c4t": lambda cpu: run_c4_family("c4t", "Tweedie", 1.5)}
+            "c4g": lambda cpu: run_c4_family("c4g", "Gamma", 2.0), "c4t": lambda cpu: run_c4_family("c4t", "Tweedie", 1.5),
+            "c4en": run_c4en}
     for name in which:
         line = runs[name](cpu)
         print(json.dumps(line), flush=True)
