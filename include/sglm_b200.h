@@ -431,7 +431,9 @@ int sglm_glm_irls_prepare_f64(const double *X, int64_t ldx, const double *y, con
  *                   calls, the way np.diff computes it — bit-exact).
  *   rolling_minmax: sglm_pp.detrend_data (:522-545): pandas rolling(window, center=True).apply(lambda_min_max) —
  *                   the window's element (W+1)//2 - 1 scaled by the window's 5 % / 95 % quantiles (linear
- *                   interpolation); NaN where the window leaves its group segment or holds a NaN.
+ *                   interpolation); NaN where the window leaves its group segment or holds a NaN or +-inf
+ *                   (pandas' rolling counts +-inf as missing).  col_moments: sd is NaN when at most ddof values
+ *                   remain (an all-NaN column with skipna, one value with ddof 1).
  * ------------------------------------------------------------------------- */
 size_t sglm_col_moments_workspace_bytes(int64_t T, int32_t C);
 int sglm_col_moments_f64(const double *X, int64_t ldx, int64_t T, int32_t C, int32_t ddof, int32_t skipna,

@@ -31,7 +31,7 @@ pp_col_partial_kernel(const double *__restrict__ X, long long ldx, long long T, 
     part[(long long)blockIdx.y * C + c] = s;
     if (!pass) cnt[(long long)blockIdx.y * C + c] = n;
 }
-// pass 0: mean[c] = sum / n, n_out[c] = n;  pass 1: std[c] = sqrt(sum / (n - ddof))
+// pass 0: mean[c] = sum / n, n_out[c] = n;  pass 1: std[c] = sqrt(sum / (n - ddof)), NaN when n <= ddof
 __global__ void __launch_bounds__(256)
 pp_col_finish_kernel(const double *__restrict__ part, const double *__restrict__ cnt, int n_chunks, int C, int pass,
                      int ddof, double *__restrict__ out, double *__restrict__ n_io) {
@@ -40,7 +40,8 @@ pp_col_finish_kernel(const double *__restrict__ part, const double *__restrict__
     double s = 0.0, n = 0.0;
     for (int k = 0; k < n_chunks; ++k) { s += part[(long long)k * C + c]; if (!pass) n += cnt[(long long)k * C + c]; }
     if (!pass) { out[c] = s / n; n_io[c] = n; }
-    else out[c] = sqrt(s / (n_io[c] - (double)ddof));
+    else out[c] = n_io[c] > (double)ddof ? sqrt(s / (n_io[c] - (double)ddof))
+                                         : __longlong_as_double(0x7ff8000000000000LL);   // pandas: NaN, not sqrt(-0.0)
 }
 __global__ void __launch_bounds__(256)
 pp_zscore_kernel(const double *__restrict__ X, long long ldx, long long T, int C, const double *__restrict__ mean,
@@ -68,9 +69,9 @@ pp_diff_kernel(const double *__restrict__ X, long long ldx, long long T_out, con
 // Rolling min-max detrending (backend/sglm_pp.py:504-545): pandas `rolling(window=W, center=True).apply(f)` with
 //   f(win) = (win[(W+1)//2 - 1] - q05) / (q95 - q05),  q = linear-interpolated quantiles of the W window values.
 // The window of output position i is x[i - W/2 .. i + (W-1)/2 ... ] = the W values starting at i - (W - 1 - (W-1)/2)
-// (pandas centring: offset (W-1)//2 to the right), it must lie inside the row's segment [seg_lo, seg_hi) and hold no
-// NaN, else the result is NaN (min_periods = W).  One CTA per output position: the window is sorted by a bitonic
-// network in shared memory (padded with +inf to a power of two).
+// (pandas centring: offset (W-1)//2 to the right), it must lie inside the row's segment [seg_lo, seg_hi) and hold
+// only finite values, else the result is NaN (min_periods = W; pandas' rolling counts +-inf as missing).  One CTA per
+// output position: the window is sorted by a bitonic network in shared memory (padded with +inf to a power of two).
 __global__ void __launch_bounds__(256)
 pp_rolling_minmax_kernel(const double *__restrict__ x, long long n, const long long *__restrict__ seg_lo,
                          const long long *__restrict__ seg_hi, int W, int Wpad, double *__restrict__ out) {
@@ -89,7 +90,7 @@ pp_rolling_minmax_kernel(const double *__restrict__ x, long long n, const long l
         __syncthreads();
         for (int k = threadIdx.x; k < Wpad; k += 256) {
             double v = __longlong_as_double(0x7ff0000000000000LL);      // +inf padding
-            if (k < W) { v = x[lo + k]; if (v != v) bad = 1; }
+            if (k < W) { v = x[lo + k]; if (!isfinite(v)) bad = 1; }
             win[k] = v;
         }
         __syncthreads();
@@ -110,15 +111,17 @@ pp_rolling_minmax_kernel(const double *__restrict__ x, long long n, const long l
                 __syncthreads();
             }
         if (threadIdx.x == 0) {
-            // numpy / pandas linear interpolation: position q (W - 1); lerp written as numpy's _lerp does it
+            // numpy / pandas linear interpolation: position q (W - 1); lerp written as numpy's _lerp does it, every
+            // product rounded before the sum (explicit _rn intrinsics: a contracted FMA rounds once and can differ
+            // from numpy in the last bit)
             auto quant = [&](double q) {
-                const double pos = q * (double)(W - 1);
+                const double pos = __dmul_rn(q, (double)(W - 1));
                 const int k = (int)floor(pos);
-                const double g = pos - (double)k;
+                const double g = __dsub_rn(pos, (double)k);
                 const double a = win[k], b2 = win[min(k + 1, W - 1)];
-                const double d = b2 - a;
-                double r = a + d * g;                                   // lerp(a, b, t) = a + (b - a) t ...
-                if (g >= 0.5) r = b2 - d * (1.0 - g);                   // ... and from the other end for t >= 0.5
+                const double d = __dsub_rn(b2, a);
+                double r = __dadd_rn(a, __dmul_rn(d, g));                                // a + (b - a) t ...
+                if (g >= 0.5) r = __dsub_rn(b2, __dmul_rn(d, __dsub_rn(1.0, g)));       // ... from b for t >= 0.5
                 return r;
             };
             const double q05 = quant(0.05), q95 = quant(0.95);
