@@ -156,8 +156,9 @@ int sglm_gram_tc_f64(const double *X, int64_t ldx, const double *Y, int64_t ldy,
                      void *stream);
 
 /* Weighted tensor-core Gram: rows of Z scaled by row_scale[t] (sqrt of a row weight: G = Z' diag(w) Z) and at
- * most max_planes digit planes per column (fewer than a column needs = digits rounded at the last plane,
- * relative error 2^-(7 max_planes)).  Replaces the X'WX of every Newton / IRLS step of the Poisson fit
+ * most max_planes digit planes per column (fewer than a column needs = digits rounded at the last plane: each
+ * value off by at most 2^(E - 7 max_planes), i.e. 2^-(7 max_planes) of the column scale 2^E > max |z|; a
+ * round-half-even tie at the last plane reaches it).  Replaces the X'WX of every Newton / IRLS step of the Poisson fit
  * (sklearn _glm/_newton_solver.py:315-359) as an APPROXIMATE Hessian; the gradient stays exact (sglm_xt_vec_f64). */
 int sglm_gram_tc_analyze_scaled_f64(const double *X, int64_t ldx, const double *Y, int64_t ldy, int32_t n_y,
                                     int64_t T, int32_t C, const double *row_scale, int32_t max_planes,

@@ -956,7 +956,8 @@ extern "C" int sglm_gram_tc_exponents(const uint64_t *colmax_bits, int32_t n_aug
 
 // Weighted form: every row t of Z = [X | Y | 1] is scaled by row_scale[t] (= sqrt of a row weight, so that the
 // Gram is Z' diag(w) Z), and at most max_planes (1..8) digit planes are kept per column: with fewer planes than
-// a column needs its digits are rounded at the last plane (relative error 2^-(7 max_planes)) — the approximate
+// a column needs its digits are rounded at the last plane (each value off by at most 2^(E - 7 max_planes), i.e.
+// 2^-(7 max_planes) of the column scale 2^E) — the approximate
 // Hessian of the Poisson Newton iteration, whose gradient stays exact.
 extern "C" int sglm_gram_tc_analyze_scaled_f64(const double *X, int64_t ldx, const double *Y, int64_t ldy,
                                                int32_t n_y, int64_t T, int32_t C, const double *row_scale,
