@@ -90,8 +90,9 @@ __device__ __forceinline__ void cta_reduce(double (&v)[K], double *scratch) {
 // blocked by 32 consecutive coordinates:
 //
 //   phase 1 (warp 0, registers + shuffles): lane l owns coordinate 32b+l and its Qw entry; the
-//     diagonal 32x32 sub-block of Q sits in shared memory (fetched with cp.async while the
-//     previous panel update runs).  The block's coordinates are visited in order, each delta is
+//     diagonal 32x32 sub-block of Q sits in shared memory (fetched with cp.async by the panel
+//     warps, idle until then, during the previous block, so that the copies are not issued from
+//     warp 0's critical path).  The block's coordinates are visited in order, each delta is
 //     broadcast with a shuffle and folded into the other lanes' Qw — the exact FMA sequence of
 //     the unblocked algorithm;
 //   phase 2 (panel warps): the rows of Q whose coefficient moved are streamed once
@@ -268,18 +269,25 @@ enet_cd_gram_kernel(const double *const *__restrict__ prob_Q, const double *cons
     }
     __syncthreads();
 
-    // asynchronous fetch of block b's diagonal sub-block, q and diag into buffer `buf` (warp 0)
-    auto fetch_block = [&](int b, int buf) {
-        const int j_l = (b << 5) + lane;
+    // asynchronous fetch of block b's diagonal sub-block, q and diag into buffer `buf`, shared by the `nt` threads
+    // t = 0..nt-1 that call it (entries past C are not copied: they are never read)
+    auto fetch_block = [&](int b, int buf, int t, int nt) {
         double *dst = blk + buf * 1024;
-        if (j_l < C) {
-#pragma unroll 8
-            for (int i = 0; i < 32; ++i) {
-                const int ji = (b << 5) + i;
-                if (ji < C) cd_cp_async8(dst + i * 32 + lane, Q + (long long)ji * ldq + j_l);
+        const int j0 = b << 5;
+        if (vec2) {
+            for (int e = t; e < 512; e += nt) {
+                const int i = e >> 4, c = (e & 15) << 1;
+                if (j0 + i < C && j0 + c < C) cd_cp_async16(dst + i * 32 + c, Q + (long long)(j0 + i) * ldq + j0 + c);
             }
-            cd_cp_async8(qd + buf * 64 + lane, q + j_l);
-            cd_cp_async8(qd + buf * 64 + 32 + lane, dg + j_l);
+        } else {
+            for (int e = t; e < 1024; e += nt) {
+                const int i = e >> 5, c = e & 31;
+                if (j0 + i < C && j0 + c < C) cd_cp_async8(dst + i * 32 + c, Q + (long long)(j0 + i) * ldq + j0 + c);
+            }
+        }
+        for (int e = t; e < 64; e += nt) {
+            const int j = j0 + (e & 31);
+            if (j < C) cd_cp_async8(qd + buf * 64 + e, (e < 32 ? q : dg) + j);
         }
         cd_cp_async_commit();
     };
@@ -290,11 +298,16 @@ enet_cd_gram_kernel(const double *const *__restrict__ prob_Q, const double *cons
         if (is_seq) {
             int b0 = 0;
             while (b0 < NBLK && act[b0] == 0u) ++b0;
-            if (b0 < NBLK) fetch_block(b0, 0);
+            if (b0 < NBLK) fetch_block(b0, 0, lane, 32);
         }
         for (int b = 0; b < NBLK; ++b) {
             const unsigned mask = act[b];
             if (mask == 0u) continue;                                     // uniform: block screened out
+            if (!is_seq) {                                                // the next active block's sub-block, into the
+                int bn = b + 1;                                           // buffer warp 0 reads next: lands during this
+                while (bn < NBLK && act[bn] == 0u) ++bn;                  // register phase and panel pass
+                if (bn < NBLK) fetch_block(bn, buf ^ 1, tid - 32, NTB);
+            }
             if (is_seq) {
                 // ---------------- phase 1: the block's coordinates, in order
                 const long long t_b = clock64();
@@ -369,10 +382,6 @@ enet_cd_gram_kernel(const double *const *__restrict__ prob_Q, const double *cons
                 if (lane == 0) { ctl[0] = nz; pmv[b] = (unsigned char)__popc(nz); }
                 n_upd += __popc(nz);
                 ++n_blk;
-                int bn = b + 1;
-                while (bn < NBLK && act[bn] == 0u) ++bn;
-                if (bn < NBLK) fetch_block(bn, buf ^ 1);                  // lands during phase 2
-                buf ^= 1;
                 t_p1 += clock64() - t_b;
             }
             __syncthreads();                                              // deltas and moved-row mask published
@@ -432,7 +441,9 @@ enet_cd_gram_kernel(const double *const *__restrict__ prob_Q, const double *cons
                     }
                 }
             }
-            __syncthreads();                                              // Qw updated
+            if (!is_seq) cd_cp_async_wait_all();
+            __syncthreads();                                              // Qw updated, next sub-block landed
+            buf ^= 1;
         }
         // ---------------- end of sweep: stopping rule / gap / screening
         if (is_seq) {
